@@ -22,6 +22,8 @@ index is built once per box under --cache.  `--workload cfg2` (100 Mbp uniform, 
   cpu_baseline  the REAL reference (oracle/_ref/bitmapperBS, compiled from /root/reference) with -t <host cores> on a
                 bounded sample of the same reads, its own mapping timer (Bitmapper_main.cpp:262)
 
+`--steps` timed steps are run in each timed loop (device-resident, end to end, cfg4).  `--dump-outputs DIR` writes what the
+end-to-end loop's last step returned to the caller (see dump_outputs); the inputs are seeded, so two builds can be compared.
 `--impl reference` times only that CPU run.  Multi-GPU (torchrun, one rank per GPU): read batches are sharded, the index is
 replicated, no collective on the data path; per-GPU work is fixed ("weak").
 """
@@ -265,6 +267,41 @@ def run_cli(exe: Path, d: Path, wl: Workload, seq_args, threads: int, out: str, 
         return None
     return float(m.group(1)), float(m.group(2)), wall
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out: Path, records, fields, lists):
+    """--dump-outputs: the per-read records of the last timed step and the per-read lists they point into, as float64 .npy
+    files (records: `<field>.npy`; lists: `<list>.npy` or `<list>_<field>.npy`, each read's entries in read order).  Offsets
+    into the lists are left out: the device hands them out in completion order.  When everything would exceed DUMP_BYTES,
+    a seeded sample of the reads (the same for the same outputs) is written; `read_index.npy` names the reads written.
+    A list with no entries among the reads written (e.g. no read handed back to the host) writes no file.
+    lists: name -> (array, first entry per read, entries per read, mask of the reads whose entries are in this array)"""
+    n = len(records)
+    m = n
+    while True:
+        idx = np.sort(np.random.default_rng(0).choice(n, m, replace=False)) if m < n else np.arange(n)
+        take = {}
+        for name, (arr, first, count, mask) in lists.items():
+            f, c = first[idx][mask[idx]].astype(np.int64), count[idx][mask[idx]].astype(np.int64)
+            take[name] = np.repeat(f - np.cumsum(c) + c, c) + np.arange(int(c.sum()))
+        nbytes = 8 * m * (len(fields) + 1) + sum(8 * len(t) * max(1, len(lists[k][0].dtype.names or ())) for k, t in take.items())
+        if nbytes <= DUMP_BYTES:
+            break
+        m //= 2
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "read_index.npy", idx.astype(np.float64))
+    for f in fields:
+        np.save(out / f"{f}.npy", records[f][idx].astype(np.float64))
+    for name, t in take.items():
+        if len(t) == 0:
+            continue
+        arr = lists[name][0][t]
+        for f in arr.dtype.names or (None,):
+            np.save(out / (f"{name}_{f}.npy" if f else f"{name}.npy"), (arr[f] if f else arr).astype(np.float64))
+    return {"dir": str(out), "reads": int(m), "of_reads": int(n), "bytes": int(nbytes), "files": sorted(f.name for f in out.glob("*.npy"))}
+
+
 def measure_cfg4(B, capi, torch, index, dev, d, scale, pairs, rank, steps, warmup, nb=4):
     """BASELINE.json configs[3] on the index that is already resident: cfg3's genome, 150 bp pairs, --pe --sensitive (the whole
     pair logic on the device: mate-range filter, hit compaction, one re-seeding round).  -> dict with the rank's device and
@@ -356,6 +393,7 @@ def main():
     ap.add_argument("--inflight", type=int, default=4, help="batches in flight in the end-to-end loop (measured: 2 -> 122, 3 -> 141, 4 -> 162, 6 -> 161 M reads/s)")
     ap.add_argument("--no-cfg4", action="store_true", help="skip the secondary cfg4 (--pe --sensitive) measurement on the same index")
     ap.add_argument("--cfg4-pairs", type=int, default=500_000, help="pairs per GPU per step of the cfg4 measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0) as .npy files under DIR")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     scale = a.scale if a.scale is not None else float(os.environ.get("BMBS_BENCH_SCALE", DEFAULT_SCALE[a.workload]))
@@ -486,12 +524,12 @@ def main():
             bb.finish()
 
     def step_download(o):
-        """-> bytes copied back"""
+        """-> (bytes copied back, the arrays the call returned)"""
         if fin_mode:
-            _, mm, fb = o[0].download_final(o[3], o[4], o[5])
-            return n_reads * capi.Final.itemsize + 2 * len(mm) + capi.Cand.itemsize * len(fb)
-        _, _, u = o[0].download(o[1], o[2])
-        return n_reads * capi.ReadResult.itemsize + u * capi.Cand.itemsize
+            got = o[0].download_final(o[3], o[4], o[5])
+            return n_reads * capi.Final.itemsize + 2 * len(got[1]) + capi.Cand.itemsize * len(got[2]), got
+        r, c, u = o[0].download(o[1], o[2])
+        return n_reads * capi.ReadResult.itemsize + u * capi.Cand.itemsize, (r, c[:u])
     clocks = ClockSampler(dev); clocks.start()
     for _ in range(max(0, a.warmup - 1)):
         step_run(batch)
@@ -537,9 +575,9 @@ def main():
         o = outs[i % NB]
         o[0].upload(flat, offs, pe=wl.pe); step_run(o[0])
         if i >= NB - 1:
-            d2h = step_download(outs[(i - (NB - 1)) % NB])
+            d2h, last = step_download(outs[(i - (NB - 1)) % NB])
     for i in range(max(0, a.steps - (NB - 1)), a.steps):
-        d2h = step_download(outs[i % NB])
+        d2h, last = step_download(outs[i % NB])
     e2e_ms = (time.perf_counter() - e0) * 1000
     barrier()
     clk = clocks.stop(t_begin, time.time())
@@ -548,6 +586,17 @@ def main():
         fin_status = np.bincount(outs[0][3]["status"], minlength=5)
     else:
         assert all(np.array_equal(outs[0][1]["state"], o[1]["state"]) for o in outs[1:])
+    dumped = None
+    if a.dump_outputs and rank == 0:
+        if fin_mode:      # finished records; mismatch positions of the reads finished on the device, windows of those handed back
+            fin, mm, fb = last
+            host = fin["status"] == capi.FIN_HOST
+            dumped = dump_outputs(Path(a.dump_outputs), fin, [f for f in capi.Final.names if f != "aux_first"],
+                                  {"mismatch_pos": (mm, fin["aux_first"], fin["n_aux"], ~host), "handed_back": (fb, fin["aux_first"], fin["n_aux"], host)})
+        else:             # per-read records and their verified windows
+            res, cand = last
+            dumped = dump_outputs(Path(a.dump_outputs), res, [f for f in capi.ReadResult.names if f not in ("first_cand", "reserved")],
+                                  {"cand": (cand, res["first_cand"], res["n_cand"], np.ones(len(res), bool))})
     h2d = int(bases + 8 * (n_reads + 1)); d2h = int(d2h)
     os.sched_setaffinity(0, full_affinity)        # the command-line runs below use every core of the box
 
@@ -557,7 +606,7 @@ def main():
         for o in outs:
             o[0].close()
         try:
-            c4 = measure_cfg4(B, capi, torch, index, dev, d, scale, a.cfg4_pairs, rank, max(a.inflight + 1, min(a.steps, 12)), a.warmup, a.inflight)
+            c4 = measure_cfg4(B, capi, torch, index, dev, d, scale, a.cfg4_pairs, rank, a.steps, a.warmup, a.inflight)
         except Exception as e:      # the headline line must not depend on the secondary measurement
             log(f"[bench r{rank}] cfg4 measurement failed: {e}")
     c4_ms = [c4["dev_ms"], c4["e2e_ms"]] if c4 else [0.0, 0.0]
@@ -632,6 +681,7 @@ def main():
         "clocks": clk,
         "stage_ms_per_step": per_step,
         "wall_ms_per_step": wall_ms / a.steps,
+        "dumped_outputs": dumped,
         "verify_gcups": gcups,
         "work_per_step": counters,
         "finishing": ({"status": {"unmapped": int(fin_status[0]), "unique_ungapped": int(fin_status[1]), "ambiguous": int(fin_status[2]), "needs_dp": int(fin_status[3]),

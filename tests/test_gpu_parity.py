@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import bitmapperbs_b200 as B
+import reference_sha256
 from bitmapperbs_b200 import capi, simulate as S
 from conftest import read_fastq, revcomp, sam_body
 from oracle_binding import OracleIndex
@@ -312,9 +313,8 @@ def test_mapper_sam_identical_to_reference_golden(golden, built, name, args, fin
 
 
 def test_live_reference_binary_agrees_on_fresh_data(built, tmp_path):
-    """fresh seeded data, larger than the golden set; compared with the real reference run on this box"""
-    if not built["ref"].exists():
-        pytest.skip("compiled reference absent")
+    """fresh seeded data, larger than the golden set; compared with the reference's SAM and mapstats: their stored digests
+    (tests/reference_sha256.py), and the reference itself where it is built"""
     chroms = S.random_genome([900000, 600000], seed=99, repeat_fraction=0.4, repeat_copies=(5, 60), repeat_len=(300, 4000))
     S.write_fasta(tmp_path / "g.fa", chroms)
     r, _ = S.simulate_reads(chroms, 12000, 125, seed=5, sub=0.025, indel=0.004, n_rate=0.002, random_qual=True, junk_fraction=0.03)
@@ -348,18 +348,20 @@ def test_live_reference_binary_agrees_on_fresh_data(built, tmp_path):
                       ("se_pbat_directional", ["--seq", "r.fq", "--pbat", "--unmapped_out"]),
                       ("pe_pbat", ["--seq1", "b.fq", "--seq2", "a.fq", "--pe", "--pbat"]),
                       ("hards_pbat", ["--seq1", "d.fq", "--seq2", "c.fq", "--pe", "--sensitive", "--pbat", "--unmapped_out"])):
-        subprocess.run([str(built["ref"]), "--search", "g.fa", *args, "-t", "1", "-o", f"cpu_{tag}.sam", "--mapstats", f"cpu_{tag}.st"],
-                       cwd=tmp_path, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         subprocess.run([str(built["bmbs"]), "--search", "g.fa", *args, "-t", "4", "-o", f"gpu_{tag}.sam", "--mapstats", f"gpu_{tag}.st"],
                        cwd=tmp_path, check=True, stderr=subprocess.DEVNULL)
-        assert sam_body(tmp_path / f"gpu_{tag}.sam") == sam_body(tmp_path / f"cpu_{tag}.sam")
-        assert (tmp_path / f"gpu_{tag}.st").read_text() == (tmp_path / f"cpu_{tag}.st").read_text()
+        body, stats = sam_body(tmp_path / f"gpu_{tag}.sam"), (tmp_path / f"gpu_{tag}.st").read_text()
+        reference_sha256.check(f"fresh_data:{tag}", b"".join(body) + stats.encode())
+        if built["ref"].exists():
+            subprocess.run([str(built["ref"]), "--search", "g.fa", *args, "-t", "1", "-o", f"cpu_{tag}.sam", "--mapstats", f"cpu_{tag}.st"],
+                           cwd=tmp_path, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            assert body == sam_body(tmp_path / f"cpu_{tag}.sam") and stats == (tmp_path / f"cpu_{tag}.st").read_text(), tag
         if "--pe" in args:      # the same pairs with every pair through the warp kernel of the pair finishing
             import os
             subprocess.run([str(built["bmbs"]), "--search", "g.fa", *args, "-t", "4", "-o", f"gpw_{tag}.sam", "--mapstats", f"gpw_{tag}.st"],
                            cwd=tmp_path, check=True, stderr=subprocess.DEVNULL, env={**os.environ, "BMBS_PE_FIN_SHORT": "0"})
-            assert sam_body(tmp_path / f"gpw_{tag}.sam") == sam_body(tmp_path / f"cpu_{tag}.sam"), tag
-            assert (tmp_path / f"gpw_{tag}.st").read_text() == (tmp_path / f"cpu_{tag}.st").read_text(), tag
+            assert sam_body(tmp_path / f"gpw_{tag}.sam") == body, tag
+            assert (tmp_path / f"gpw_{tag}.st").read_text() == stats, tag
 
 
 def test_mapper_wide_suffix_array_gzip_input_and_two_gpus(golden, built, tmp_path):
@@ -436,10 +438,13 @@ def test_mapper_bam_output_holds_the_same_records(golden, built, name, args):
         assert (r["name"], r["flag"], r["rid"], r["pos"], r["mapq"], r["cigar"], r["seq"], r["qual"], r["tags"]) == \
                (f[0], int(f[1]), rid[f[2]], int(f[3]) - 1, int(f[4]), f[5], f[9], f[10], f[11:])
         assert r["npos"] == int(f[7]) - 1 and r["tlen"] == int(f[8])
-    # and byte for byte what the reference's own writer (the stock reference linked with its vendored, patched htslib) puts out
+    # and byte for byte what the reference's own writer (the stock reference linked with its vendored, patched htslib) puts out:
+    # its stored digest, and the reference itself where it is built
+    from test_host_bam import bam_payload
+    gt, gd, gr = bam_payload(golden / "gpu.bam")
+    reference_sha256.check(f"bmbs_bam:{name}", gd + gr)
     ref = ROOT_DIR / "oracle/_ref/bitmapperBS_bam"
     if ref.exists():
-        from test_host_bam import bam_payload
         subprocess.run([str(ref), "--search", "genome.fa", *args, "-t", "1", "--bam", "-o", "ref.bam"], cwd=golden, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-        gt, gd, gr = bam_payload(golden / "gpu.bam"); rt, rd, rr = bam_payload(golden / "ref.bam")
+        rt, rd, rr = bam_payload(golden / "ref.bam")
         assert gd == rd and gr == rr

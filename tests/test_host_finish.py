@@ -1,12 +1,14 @@
 """Host finishing code of the product (bitmapperbs_b200/csrc/host/mapper.hpp: vote-ordered reduction, pair pick, CIGAR
 refinement, MAPQ, SAM text; finish_single_final / finish_pair_final behind the finished records), on the CPU: fed with the ORACLE's per-read records -- the same arrays the GPU library returns
 (tests/test_gpu_parity.py) -- its SAM must equal the golden SAM of the real reference, record for record, and the
---mapstats counters with it.  Covers single end, paired end fast and sensitive, and --unmapped_out against the live reference."""
+--mapstats counters with it.  Covers single end, paired end fast and sensitive, and --unmapped_out, --ambiguous_out and --pbat
+against the reference's output (tests/reference_sha256.py)."""
 import subprocess
 from pathlib import Path
 
 import pytest
 
+import reference_sha256
 from conftest import sam_body
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -40,13 +42,15 @@ def test_host_finish_matches_reference_golden(golden, harness, name, mode, files
 @pytest.mark.parametrize("mode,files", [("se", ["se100.fq"]), ("sef", ["se100.fq"]), ("pe", ["pe100h_1.fq", "pe100h_2.fq"]), ("pes", ["pe100h_1.fq", "pe100h_2.fq"]),
                                         ("pef", ["pe100h_1.fq", "pe100h_2.fq"]), ("pesf", ["pe100h_1.fq", "pe100h_2.fq"])])
 def test_unmapped_out_matches_live_reference(golden, built, harness, mode, files):
-    if not built["ref"].exists():
-        pytest.skip("compiled reference absent")
-    args = ["--seq", files[0]] if mode in ("se", "sef") else ["--seq1", files[0], "--seq2", files[1], "--pe"] + (["--sensitive"] if mode in ("pes", "pesf") else [])
-    subprocess.run([str(built["ref"]), "--search", "genome.fa", *args, "--unmapped_out", "-t", "1", "-o", f"ref_un_{mode}.sam"],
-                   cwd=golden, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    """against the reference's SAM: its stored digest, and the live reference where it is built"""
     subprocess.run([str(harness), mode, "genome.fa", f"hf_un_{mode}.sam", *files, "--unmapped_out"], cwd=golden, check=True, capture_output=True)
-    assert sam_body(golden / f"hf_un_{mode}.sam") == sam_body(golden / f"ref_un_{mode}.sam")
+    ours = sam_body(golden / f"hf_un_{mode}.sam")
+    reference_sha256.check(f"host_finish_unmapped_out:{mode}", b"".join(ours))
+    if built["ref"].exists():
+        args = ["--seq", files[0]] if mode in ("se", "sef") else ["--seq1", files[0], "--seq2", files[1], "--pe"] + (["--sensitive"] if mode in ("pes", "pesf") else [])
+        subprocess.run([str(built["ref"]), "--search", "genome.fa", *args, "--unmapped_out", "-t", "1", "-o", f"ref_un_{mode}.sam"],
+                       cwd=golden, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        assert ours == sam_body(golden / f"ref_un_{mode}.sam")
 
 
 @pytest.mark.parametrize("mode,files,flags", [("pe", ["pe100h_1.fq", "pe100h_2.fq"], ["--ambiguous_out"]), ("pes", ["pe100h_1.fq", "pe100h_2.fq"], ["--ambiguous_out", "--unmapped_out"]),
@@ -57,9 +61,8 @@ def test_unmapped_out_matches_live_reference(golden, built, harness, mode, files
                                               ("sef", ["se100_rc.fq"], ["--pbat", "--unmapped_out"]), ("sef", ["se100.fq"], ["--pbat", "--unmapped_out"])])
 def test_flag_rows_match_live_reference(golden, built, harness, mode, files, flags):
     """--ambiguous_out (paired end), --pbat (single end on reverse-complemented reads and on directional ones; paired end with
-    the files swapped so that pairs still map) and --unmapped_out with them, against the live reference"""
-    if not built["ref"].exists():
-        pytest.skip("compiled reference absent")
+    the files swapped so that pairs still map) and --unmapped_out with them, against the reference's SAM (its stored digest, and the
+    live reference where it is built)"""
     if not (golden / "se100_rc.fq").exists():
         comp = bytes.maketrans(b"ACGTacgt", b"TGCAtgca")
         ls = (golden / "se100.fq").read_bytes().split(b"\n")
@@ -68,8 +71,11 @@ def test_flag_rows_match_live_reference(golden, built, harness, mode, files, fla
                 o.write(ls[i] + b"\n" + ls[i + 1].translate(comp)[::-1] + b"\n+\n" + ls[i + 3][::-1] + b"\n")
     tag = mode + "_" + "_".join(f.strip("-") for f in flags) + "_" + files[0].split(".")[0]
     args = ["--seq", files[0]] if mode in ("se", "sef") else ["--seq1", files[0], "--seq2", files[1], "--pe"] + (["--sensitive"] if mode in ("pes", "pesf") else [])
-    subprocess.run([str(built["ref"]), "--search", "genome.fa", *args, *flags, "-t", "1", "-o", f"ref_{tag}.sam"],
-                   cwd=golden, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     subprocess.run([str(harness), mode, "genome.fa", f"hf_{tag}.sam", *files, *flags], cwd=golden, check=True, capture_output=True)
-    ref = sam_body(golden / f"ref_{tag}.sam")
-    assert len(ref) > 100 and sam_body(golden / f"hf_{tag}.sam") == ref
+    ours = sam_body(golden / f"hf_{tag}.sam")
+    assert len(ours) > 100
+    reference_sha256.check(f"host_finish_flags:{tag}", b"".join(ours))
+    if built["ref"].exists():
+        subprocess.run([str(built["ref"]), "--search", "genome.fa", *args, *flags, "-t", "1", "-o", f"ref_{tag}.sam"],
+                       cwd=golden, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        assert ours == sam_body(golden / f"ref_{tag}.sam")

@@ -1,18 +1,19 @@
 """SURVEY.md 8f-1 (CIGAR + score): host/postprocess.hpp refine_alignment -- the CPU restatement the oracle CLI and the parity
 tests use -- against the REFERENCE's own fast_recalculate_bs_Cigar (ksw.cpp:2578-3148, compiled into oracle/_ref/libref_ksw.so)
 on seeded random alignments: substitutions only, insertions, deletions, N in read and window, bisulfite T/C pairs, both
-strands, reversed qualities (mate 2), quality-dependent penalties, non-default scoring.  Bit-exact: start, end, NM, score, CIGAR."""
+strands, reversed qualities (mate 2), quality-dependent penalties, non-default scoring.  Bit-exact: start, end, NM, score, CIGAR.
+Where the reference is not built, its results are compared through their stored digest (tests/reference_sha256.py)."""
 import ctypes as C
 from pathlib import Path
 
 import numpy as np
 import pytest
 
+import reference_sha256
 from oracle_binding import lib
 
 ROOT = Path(__file__).resolve().parent.parent
 REF = ROOT / "oracle/_ref/libref_ksw.so"
-pytestmark = pytest.mark.skipif(not REF.exists(), reason="oracle/_ref not built (needs /root/reference)")
 
 
 def make_case(rng, L, k, n_sub, n_ins, n_del, n_frac):
@@ -59,10 +60,11 @@ def edit_end(win, read, k):
 @pytest.mark.parametrize("seed,L,k,scoring", [(1, 100, 8, (6, 2, 1, 5, 3, 33)), (2, 150, 12, (6, 2, 1, 5, 3, 33)), (3, 60, 4, (6, 2, 1, 5, 3, 33)),
                                               (4, 150, 12, (4, 1, 2, 3, 1, 33)), (5, 120, 9, (6, 2, 1, 5, 3, 64))])
 def test_refine_matches_reference(seed, L, k, scoring):
-    ref = C.CDLL(str(REF)); orc = lib()
+    ref = C.CDLL(str(REF)) if REF.exists() else None
+    orc = lib()
     rng = np.random.default_rng(seed)
     mp_max, mp_min, n_pen, go, ge, qb = scoring
-    n = 0
+    results = []
     for case in range(400):
         n_ins, n_del = int(rng.integers(0, 3)), int(rng.integers(0, 3))
         n_sub = int(rng.integers(0, 4))
@@ -74,12 +76,15 @@ def test_refine_matches_reference(seed, L, k, scoring):
             continue
         for forward in (1, 0):
             for rq in (0, 1):
-                s1, e1, n1, sc1 = C.c_int(), C.c_uint64(), C.c_uint(), C.c_int(); c1 = C.create_string_buffer(4096)
                 s2, e2, n2, sc2 = C.c_int(), C.c_uint64(), C.c_uint(), C.c_int(); c2 = C.create_string_buffer(4096)
-                ref.ref_cigar(win, len(win), read, L, k, end, err, forward, mp_max, mp_min, n_pen, go, ge, qual, rq, qb,
-                              C.byref(s1), C.byref(e1), C.byref(n1), C.byref(sc1), c1)
                 orc.orc_refine(win, len(win), read, L, k, end, err, forward, qual, rq, mp_max, mp_min, n_pen, go, ge, qb,
                                C.byref(s2), C.byref(e2), C.byref(n2), C.byref(sc2), c2, 4096)
-                assert (s1.value, e1.value, n1.value, sc1.value, c1.value) == (s2.value, e2.value, n2.value, sc2.value, c2.value), (case, forward, rq, read, win)
-                n += 1
-    assert n > 800
+                got = (s2.value, e2.value, n2.value, sc2.value, c2.value)
+                if ref:
+                    s1, e1, n1, sc1 = C.c_int(), C.c_uint64(), C.c_uint(), C.c_int(); c1 = C.create_string_buffer(4096)
+                    ref.ref_cigar(win, len(win), read, L, k, end, err, forward, mp_max, mp_min, n_pen, go, ge, qual, rq, qb,
+                                  C.byref(s1), C.byref(e1), C.byref(n1), C.byref(sc1), c1)
+                    assert (s1.value, e1.value, n1.value, sc1.value, c1.value) == got, (case, forward, rq, read, win)
+                results.append(got)
+    assert len(results) > 800
+    reference_sha256.check(f"refine:{seed}", repr(results).encode())
