@@ -475,7 +475,7 @@ extern "C" int bmbs_batch_create(bmbs_index* idx, int dev, size_t max_reads, siz
   A(dalloc(b, &b->d_ascii, max_bases + 64)); A(dalloc(b, &b->d_offsets, R));
   A(dalloc(b, &v.codes, 4 * (max_bases / 32 + 2 * R + 64))); A(dalloc(b, &v.rplanes, max_bases / 32 + 2 * R + 64)); A(dalloc(b, &v.len, R)); A(dalloc(b, &v.first_c, R)); A(dalloc(b, &v.kk, R));
   A(dalloc(b, &v.state, R)); A(dalloc(b, &v.flags, R)); A(dalloc(b, &v.one_mm, R)); A(dalloc(b, &v.site0, R));
-  A(dalloc(b, &v.ph_off, R)); A(dalloc(b, &v.ph_first_len, R)); A(dalloc(b, &v.ph_seed_id, R)); A(dalloc(b, &v.list2, R)); A(dalloc(b, &v.list3, R)); A(dalloc(b, &v.list_count, 4));
+  A(dalloc(b, &v.list_count, 4));
   A(dalloc(b, &v.bk, 5 * R)); A(dalloc(b, &v.first_cands, R)); A(dalloc(b, &v.list4, R)); A(dalloc(b, &v.res_first, R)); A(dalloc(b, &v.res_n, R));
   A(dalloc(b, &v.ntask, R)); A(dalloc(b, &v.ncand, R)); A(dalloc(b, &v.coff, R)); A(dalloc(b, &v.tasks, (size_t)MAX_TASKS * max_reads));
   A(dalloc(b, &v.slot_row, S)); A(dalloc(b, &v.slot_adj, S)); A(dalloc(b, &v.slot_read, S)); A(dalloc(b, &v.cand, S)); A(dalloc(b, &v.vcnt, S));
@@ -537,6 +537,24 @@ int run_scan(bmbs_batch* b, const u32* in, u32 n, u32* out, u64* total, u64 cap,
   b->launches += 3;
   return 0;
 }
+
+// The candidates of a seeding round, from the seed tasks of every read: offsets of the candidate slots, the sites of the
+// seeds' rows, then the votes per read (votes_classify finishes short segments, the other five kernels sort longer ones by
+// size class).  `located`, when given, is recorded after expand_locate.
+int launch_candidates(bmbs_batch* b, const DevIndex& ix, const BatchView& v, cudaEvent_t located) {
+  const int n = v.n_reads;
+  cudaStream_t s = b->stream;
+  run_scan(b, v.ncand, (u32)n, v.coff, v.totals, v.slot_cap, 2u);
+  expand_locate<<<(n + 127) / 128, 128, 0, s>>>(ix, v); ++b->launches;
+  if (located) CU(cudaEventRecord(located, s));
+  votes_classify<<<(n + 127) / 128, 128, 0, s>>>(v); ++b->launches;
+  votes_sort<32><<<b->sm_count * 4, 128, 0, s>>>(v); ++b->launches;
+  votes_mid<<<b->sm_count * 8, 128, 0, s>>>(v); ++b->launches;
+  votes_big1k<<<b->sm_count * 8, 128, 0, s>>>(v); ++b->launches;
+  votes_big<<<b->sm_count * 4, 256, 4096 * sizeof(u64), s>>>(v, 4096u, 0u, 4096u); ++b->launches;
+  votes_big<<<b->sm_count * 2, BIG_THREADS, BIG_SMEM_ELEMS * sizeof(u64), s>>>(v, (u32)BIG_SMEM_ELEMS, 8192u, 0xFFFFFFFFu); ++b->launches;
+  return BMBS_OK;
+}
 }  // namespace
 
 extern "C" int bmbs_batch_run(bmbs_batch* b, const bmbs_params* prm) {
@@ -561,31 +579,17 @@ extern "C" int bmbs_batch_run(bmbs_batch* b, const bmbs_params* prm) {
     // read chunks staged per thread in shared memory: max_len/32 + 2 chunks of 16 bytes, at most 12 (longer reads: the rest from global memory)
     const u32 plane_cap = (u32)std::min(b->max_len / 32 + 2, 12);
     const size_t seed_smem = (size_t)plane_cap * SEED_BLOCK * sizeof(uint4);
-    if (!getenv("BMBS_SEED_PHASES")) {
-      // one persistent kernel: a lane per read, one dependent access per loop iteration, finished lanes take the next read
-      if (plane_cap != b->seed_plane_cap) {      // resident blocks: registers and the staged read chunks decide
-        int per_sm = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, seed_reads, SEED_BLOCK, seed_smem) == cudaSuccess && per_sm > 0) b->seed_blocks_per_sm = per_sm;
-        if (const char* e = getenv("BMBS_SEED_BLOCKS")) b->seed_blocks_per_sm = std::max(1, atoi(e));
-        b->seed_plane_cap = plane_cap;
-      }
-      const int seed_blocks = std::min((n + SEED_BLOCK - 1) / SEED_BLOCK, b->sm_count * b->seed_blocks_per_sm);
-      seed_reads<<<seed_blocks, SEED_BLOCK, seed_smem, s>>>(ix, v, plane_cap); ++b->launches;
-    } else {      // the three phase kernels (one loop nest per read), kept for comparison
-      seed_first<<<(n + 127) / 128, SEED_BLOCK, seed_smem, s>>>(ix, v, plane_cap); ++b->launches;
-      seed_second<<<(n + 127) / 128, SEED_BLOCK, seed_smem, s>>>(ix, v, plane_cap); ++b->launches;
-      seed_rest<<<(n + 127) / 128, SEED_BLOCK, seed_smem, s>>>(ix, v, plane_cap); ++b->launches;
+    // one persistent kernel: a lane per read, one dependent access per loop iteration, finished lanes take the next read
+    if (plane_cap != b->seed_plane_cap) {      // resident blocks: registers and the staged read chunks decide
+      int per_sm = 0;
+      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, seed_reads, SEED_BLOCK, seed_smem) == cudaSuccess && per_sm > 0) b->seed_blocks_per_sm = per_sm;
+      if (const char* e = getenv("BMBS_SEED_BLOCKS")) b->seed_blocks_per_sm = std::max(1, atoi(e));
+      b->seed_plane_cap = plane_cap;
     }
+    const int seed_blocks = std::min((n + SEED_BLOCK - 1) / SEED_BLOCK, b->sm_count * b->seed_blocks_per_sm);
+    seed_reads<<<seed_blocks, SEED_BLOCK, seed_smem, s>>>(ix, v, plane_cap); ++b->launches;
     CU(cudaEventRecord(b->ev[2], s));
-    run_scan(b, v.ncand, (u32)n, v.coff, v.totals, v.slot_cap, 2u);
-    expand_locate<<<(n + 127) / 128, 128, 0, s>>>(ix, v); ++b->launches;
-    CU(cudaEventRecord(b->ev[3], s));
-    votes_classify<<<(n + 127) / 128, 128, 0, s>>>(v); ++b->launches;
-    votes_sort<32><<<b->sm_count * 4, 128, 0, s>>>(v); ++b->launches;
-    votes_mid<<<b->sm_count * 8, 128, 0, s>>>(v); ++b->launches;
-    votes_big1k<<<b->sm_count * 8, 128, 0, s>>>(v); ++b->launches;
-    votes_big<<<b->sm_count * 4, 256, 4096 * sizeof(u64), s>>>(v, 4096u, 0u, 4096u); ++b->launches;
-    votes_big<<<b->sm_count * 2, BIG_THREADS, BIG_SMEM_ELEMS * sizeof(u64), s>>>(v, (u32)BIG_SMEM_ELEMS, 8192u, 0xFFFFFFFFu); ++b->launches;
+    if (int rc = launch_candidates(b, ix, v, b->ev[3])) return rc;
     CU(cudaEventRecord(b->ev[4], s));
     if (b->pe && !v.sensitive) { filter_pairs_kernel<<<(n / 2 + 127) / 128, 128, 0, s>>>(v); ++b->launches; }
     CU(cudaEventRecord(b->ev[5], s));
@@ -599,14 +603,7 @@ extern "C" int bmbs_batch_run(bmbs_batch* b, const bmbs_params* prm) {
       reseed_clear<<<(n + 255) / 256, 256, 0, s>>>(v); ++b->launches;
       BatchView w = v; w.round = 1;
       seed_reseed<<<b->sm_count * 8, SEED_BLOCK, seed_smem, s>>>(ix, w, plane_cap); ++b->launches;
-      run_scan(b, w.ncand, (u32)n, w.coff, w.totals, w.slot_cap, 2u);
-      expand_locate<<<(n + 127) / 128, 128, 0, s>>>(ix, w); ++b->launches;
-      votes_classify<<<(n + 127) / 128, 128, 0, s>>>(w); ++b->launches;
-      votes_sort<32><<<b->sm_count * 4, 128, 0, s>>>(w); ++b->launches;
-      votes_mid<<<b->sm_count * 8, 128, 0, s>>>(w); ++b->launches;
-      votes_big1k<<<b->sm_count * 8, 128, 0, s>>>(w); ++b->launches;
-      votes_big<<<b->sm_count * 4, 256, 4096 * sizeof(u64), s>>>(w, 4096u, 0u, 4096u); ++b->launches;
-      votes_big<<<b->sm_count * 2, BIG_THREADS, BIG_SMEM_ELEMS * sizeof(u64), s>>>(w, (u32)BIG_SMEM_ELEMS, 8192u, 0xFFFFFFFFu); ++b->launches;
+      if (int rc = launch_candidates(b, ix, w, nullptr)) return rc;
       sens_reseed_filter<<<b->sm_count * 4, 128, 0, s>>>(w); ++b->launches;
       run_scan(b, w.nv, (u32)n, w.voff, w.totals + 1, w.slot_cap, 4u, w.totals + 2);
       gather_work<<<(n + 127) / 128, 128, 0, s>>>(w); ++b->launches;
