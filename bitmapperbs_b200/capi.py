@@ -50,7 +50,8 @@ EXPORTS = ["bmbs_index_load", "bmbs_index_free", "bmbs_index_genome_length", "bm
            "bmbs_params_default", "bmbs_map_batch_se", "bmbs_map_batch_pe", "bmbs_verify", "bmbs_batch_create", "bmbs_batch_free",
            "bmbs_batch_upload", "bmbs_batch_run", "bmbs_batch_download", "bmbs_batch_sync", "bmbs_batch_timings",
            "bmbs_batch_counters", "bmbs_batch_launches", "bmbs_batch_verify", "bmbs_batch_download_verify", "bmbs_ubench_int_pipe", "bmbs_pinned_alloc", "bmbs_pinned_free", "bmbs_ubench_random_sectors",
-           "bmbs_refiner_create", "bmbs_refiner_free", "bmbs_refine", "bmbs_batch_finish", "bmbs_batch_download_final", "bmbs_batch_finish_counters", "bmbs_debug_sort_order", "bmbs_refiner_kernel_ms", "bmbs_batch_output_sizes"]
+           "bmbs_refiner_create", "bmbs_refiner_free", "bmbs_refine", "bmbs_batch_finish", "bmbs_batch_download_final", "bmbs_batch_finish_counters", "bmbs_debug_sort_order", "bmbs_refiner_kernel_ms", "bmbs_batch_output_sizes",
+           "bmbs_batch_grid"]
 
 
 def load_library():
@@ -82,6 +83,7 @@ def load_library():
     L.bmbs_batch_timings.argtypes = [vp, C.POINTER(C.c_float)]
     L.bmbs_batch_counters.argtypes = [vp, u64p]
     L.bmbs_batch_launches.argtypes = [vp]
+    L.bmbs_batch_grid.argtypes = [vp, C.POINTER(C.c_uint32)]
     L.bmbs_batch_verify.argtypes = [vp, vp, vp, C.c_size_t, C.c_double]
     L.bmbs_batch_download_verify.argtypes = [vp, vp, vp, C.c_size_t]
     L.bmbs_ubench_int_pipe.argtypes = [C.c_int, C.POINTER(C.c_double)]
@@ -288,6 +290,13 @@ class Batch:
 
     def launches(self):
         return int(self._L.bmbs_batch_launches(self._h))
+
+    def grid(self):
+        """test entry: [SMs the grids are sized for, seed_reads blocks of the last run, verify_windows blocks of its last
+        launch, their block size]"""
+        g = (C.c_uint32 * 4)()
+        _check(self._L.bmbs_batch_grid(self._h, g))
+        return [int(x) for x in g]
 
     def close(self):
         if self._h:

@@ -121,6 +121,7 @@ int load_files(const std::string& prefix, HostIndex& h) {
 
 struct DeviceCopy {
   int dev = 0; DevIndex view{}; size_t bytes = 0;
+  int grid_sms = 148;        // SMs the persistent and grid-stride launches of batches and refiners are sized for (BMBS_GRID_SMS)
   void *occ = nullptr, *flag = nullptr, *hash = nullptr, *ssa = nullptr, *planes = nullptr, *dsa_lo = nullptr, *dsa_hi = nullptr, *ktab = nullptr, *chroms = nullptr;
 };
 
@@ -288,6 +289,13 @@ extern "C" int bmbs_index_load(const char* index_prefix, const int* devices, int
     cudaError_t e = cudaSetDevice(c.dev);
     cudaDeviceProp prop; if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, c.dev);
     const int grid = e == cudaSuccess ? prop.multiProcessorCount * 16 : 1;
+    // BMBS_GRID_SMS=n sizes the persistent and grid-stride launches of every batch and refiner on this copy for min(n, SMs) SMs
+    // (tests: a batch of a few thousand reads then gives each lane, warp and block of those kernels many items in turn, so
+    // the reset of per-item state between items runs everywhere)
+    if (e == cudaSuccess) {
+      c.grid_sms = prop.multiProcessorCount;
+      if (const char* gs = getenv("BMBS_GRID_SMS")) { const int g = atoi(gs); if (g >= 1) c.grid_sms = std::min(g, c.grid_sms); }
+    }
     // raw file arrays -> device (16 zero words of slack behind bwt and sa_flag, as the re-layout reads a little past the end)
     void *r_bwt = nullptr, *r_high = nullptr, *r_flag = nullptr, *r_hi = nullptr, *r_lo = nullptr, *r_pac = nullptr;
     auto raw = [&](void** p, const void* src, size_t bytes, size_t slack) -> cudaError_t {
@@ -408,6 +416,7 @@ struct bmbs_batch {
   size_t mism_cap = 0, fb_cap = 0; bool finished = false;
   int n_reads = 0, pe = 0, max_len = 0, launches = 0, sm_count = 148, seed_blocks_per_sm = 8; u32 seed_plane_cap = 0;
   u32 pe_short = 48;             // pairs with more hits than this go to the warp kernel of the pair finishing (BMBS_PE_FIN_SHORT: tests)
+  u32 seed_grid = 0, verify_grid = 0, verify_block = 0;   // as launched last (bmbs_batch_grid)
   bool ran = false;
 };
 
@@ -426,6 +435,7 @@ void launch_verify(bmbs_batch* b, double e_rate, cudaStream_t s, const DevIndex&
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, verify_windows, bd, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
   if (per_sm > 12) per_sm = 12;
   verify_windows<<<b->sm_count * per_sm, bd, smem, s>>>(ix, v, std::max(nch2, 1)); ++b->launches;
+  b->verify_grid = (u32)(b->sm_count * per_sm); b->verify_block = (u32)bd;
 }
 // device arrays of a batch are carved out of one slab (one cudaMalloc per batch context): requests are recorded first
 struct SlabRequest { void** slot; size_t bytes; };
@@ -465,7 +475,7 @@ extern "C" int bmbs_batch_create(bmbs_index* idx, int dev, size_t max_reads, siz
   CU(cudaSetDevice(dev));
   bmbs_batch* b = new bmbs_batch();
   b->idx = idx; b->copy = c; b->dev = dev; b->max_reads = max_reads; b->max_bases = max_bases; b->cand_cap = cand_cap;
-  cudaDeviceProp prop; cudaGetDeviceProperties(&prop, dev); b->sm_count = prop.multiProcessorCount;
+  b->sm_count = c->grid_sms;
   if (const char* e = getenv("BMBS_PE_FIN_SHORT")) b->pe_short = (u32)std::max(0, atoi(e));
   BatchView& v = b->v;
   const size_t R = max_reads + 2, S = cand_cap + 64;
@@ -588,6 +598,7 @@ extern "C" int bmbs_batch_run(bmbs_batch* b, const bmbs_params* prm) {
     }
     const int seed_blocks = std::min((n + SEED_BLOCK - 1) / SEED_BLOCK, b->sm_count * b->seed_blocks_per_sm);
     seed_reads<<<seed_blocks, SEED_BLOCK, seed_smem, s>>>(ix, v, plane_cap); ++b->launches;
+    b->seed_grid = (u32)seed_blocks;
     CU(cudaEventRecord(b->ev[2], s));
     if (int rc = launch_candidates(b, ix, v, b->ev[3])) return rc;
     CU(cudaEventRecord(b->ev[4], s));
@@ -614,6 +625,7 @@ extern "C" int bmbs_batch_run(bmbs_batch* b, const bmbs_params* prm) {
     finalize_reads<<<(n + 255) / 256, 256, 0, s>>>(v); ++b->launches;
   } else {
     for (int i = 1; i <= 7; ++i) CU(cudaEventRecord(b->ev[i], s));
+    b->seed_grid = 0;
   }
   CU(cudaEventRecord(b->ev[8], s));
   CU(cudaMemcpyAsync(b->h_small, v.totals, 2 * 8, cudaMemcpyDeviceToHost, s));
@@ -741,6 +753,14 @@ extern "C" int bmbs_batch_counters(bmbs_batch* b, uint64_t c[8]) {
 }
 
 extern "C" int bmbs_batch_launches(bmbs_batch* b) { return b ? b->launches : 0; }
+
+// test entry: the grids as launched, so that a test can see how many items each lane / thread of the persistent and grid-stride
+// kernels had to take
+extern "C" int bmbs_batch_grid(bmbs_batch* b, uint32_t g[4]) {
+  if (!b || !g) return fail(BMBS_ERR_ARG, "bad argument");
+  g[0] = (uint32_t)b->sm_count; g[1] = b->seed_grid; g[2] = b->verify_grid; g[3] = b->verify_block;
+  return BMBS_OK;
+}
 
 extern "C" void* bmbs_pinned_alloc(size_t bytes) { void* p = nullptr; return cudaMallocHost(&p, bytes ? bytes : 1) == cudaSuccess ? p : nullptr; }
 extern "C" void bmbs_pinned_free(void* p) { if (p) cudaFreeHost(p); }
@@ -917,7 +937,7 @@ extern "C" int bmbs_refiner_create(bmbs_index* idx, int dev, bmbs_refiner** out)
   bmbs_refiner* r = new bmbs_refiner();
   r->idx = idx; r->copy = copy; r->dev = dev;
   CU(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking));
-  { cudaDeviceProp prop; if (cudaGetDeviceProperties(&prop, dev) == cudaSuccess) r->sm_count = prop.multiProcessorCount; }
+  r->sm_count = copy->grid_sms;
   cudaFuncSetAttribute(refine_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, RW_WARPS * 1000 * (int)sizeof(uint4));
   CU(cudaMalloc(&r->d_total, 8));
   CU(cudaMallocHost(&r->h_total, 8));

@@ -151,6 +151,10 @@ void bmbs_pinned_free(void* p);
 int bmbs_ubench_random_sectors(int dev, size_t bytes, double* sectors_per_second);
 /* number of kernels launched by the last bmbs_batch_run */
 int bmbs_batch_launches(bmbs_batch* b);
+/* test entry: the grids as launched (host values): [0] SMs the persistent and grid-stride launches are sized for (the device's
+ * count, or fewer with BMBS_GRID_SMS=n at index load) [1] seed_reads blocks of the last bmbs_batch_run [2] verify_windows blocks
+ * of its last launch [3] their block size */
+int bmbs_batch_grid(bmbs_batch* b, uint32_t g[4]);
 
 
 /* ---- finished single-end records (SURVEY.md 8a V3 + 8f-1): reduction, ungapped CIGAR, coordinates on the device -----

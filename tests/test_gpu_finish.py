@@ -49,9 +49,28 @@ def assert_same_final(gfin, gmism, ofin, omism, res, cand, allow_host=0):
         assert n == res["n_cand"][r]
 
 
-@pytest.fixture(scope="module")
-def idx_pair(golden):
-    ix = B.Index(golden / "genome.fa.index"); ox = OracleIndex(golden / "genome.fa.index")
+# index environments: the device's grid, and every persistent and grid-stride launch sized for one SM -- each warp or block of
+# finish_long, finish_huge, finish_sorted and finish_pe_long then takes many reads in turn
+GRIDS = {"default": {}, "small_grid": {"BMBS_GRID_SMS": "1"}}
+
+
+def load_index(prefix, env):
+    import os
+    old = {k: os.environ.get(k) for k in env}
+    os.environ.update(env)
+    try:
+        return B.Index(prefix)
+    finally:
+        for k, v in old.items():
+            if v is None:
+                os.environ.pop(k, None)
+            else:
+                os.environ[k] = v
+
+
+@pytest.fixture(scope="module", params=list(GRIDS))
+def idx_pair(golden, request):
+    ix = load_index(golden / "genome.fa.index", GRIDS[request.param]); ox = OracleIndex(golden / "genome.fa.index")
     yield ix, ox
     ix.close()
 
@@ -82,16 +101,18 @@ def test_finished_records_on_high_copy_repeats(built, tmp_path, amb_out):
     g, st = S.concat_genome(chroms)
     m1, _ = S.simulate_fast(g, st, 8000, 150, 17, paired=False, indel_reads=0.2)
     reads = [bytes(r) for r in m1]
-    ix = B.Index(tmp_path / "g.fa.index"); ox = OracleIndex(tmp_path / "g.fa.index")
-    try:
-        res, cand, fin, mism, fb, c = device_finish(ix, reads, capi.default_params(ambiguous_out=amb_out))
-        ofin, omism = ox.finish_se(reads, res, cand, ambiguous_out=bool(amb_out))
-        n = res["n_cand"][res["state"] == B.VERIFY]
-        assert (n > 16).sum() > 100 and (n > 256).any()
-        assert c["reads_sort_replayed"] > 10, c
-        assert_same_final(fin, mism, ofin, omism, res, cand, allow_host=(n > 2048).sum())
-    finally:
-        ix.close()
+    ox = OracleIndex(tmp_path / "g.fa.index")
+    for grid, env in GRIDS.items():
+        ix = load_index(tmp_path / "g.fa.index", env)
+        try:
+            res, cand, fin, mism, fb, c = device_finish(ix, reads, capi.default_params(ambiguous_out=amb_out))
+            ofin, omism = ox.finish_se(reads, res, cand, ambiguous_out=bool(amb_out))
+            n = res["n_cand"][res["state"] == B.VERIFY]
+            assert (n > 16).sum() > 100 and (n > 256).any(), grid
+            assert c["reads_sort_replayed"] > 10, (grid, c)
+            assert_same_final(fin, mism, ofin, omism, res, cand, allow_host=(n > 2048).sum())
+        finally:
+            ix.close()
 
 
 def test_device_sort_replay_equals_std_sort():
@@ -179,18 +200,20 @@ def test_finished_pairs_on_high_copy_repeats(built, tmp_path, sensitive):
     m1, m2 = S.simulate_fast(g, st, 5000, 120, 23)
     comp = bytes.maketrans(b"ACGT", b"TGCA")
     mates = [x for a, b in zip(m1, m2) for x in (bytes(a), bytes(b).translate(comp)[::-1])]
-    ix = B.Index(tmp_path / "g.fa.index"); ox = OracleIndex(tmp_path / "g.fa.index")
-    try:
-        for amb_out in (0, 1):
-            p = capi.default_params(sensitive=sensitive, ambiguous_out=amb_out)
-            res, cand, fin, mism, c = device_finish_pe(ix, mates, p)
-            n = res["n_cand"][0::2] + res["n_cand"][1::2]
-            assert (n > 48).sum() > 20 and (n > 100).any(), n.max()       # (fast mode: filter_pairs has already thinned the lists)
-            ofin, omism = ox.finish_pe(mates, res, cand, sensitive=bool(sensitive), ambiguous_out=bool(amb_out))
-            assert_same_pairs(fin, mism, ofin, omism)
-            if not amb_out:
-                assert (fin["status"][0::2] == capi.FIN_AMBIGUOUS).sum() > 5
-            else:
-                assert (fin["flags"][0::2] & 2).astype(bool).sum() > 5
-    finally:
-        ix.close()
+    ox = OracleIndex(tmp_path / "g.fa.index")
+    for grid, env in GRIDS.items():
+        ix = load_index(tmp_path / "g.fa.index", env)
+        try:
+            for amb_out in (0, 1):
+                p = capi.default_params(sensitive=sensitive, ambiguous_out=amb_out)
+                res, cand, fin, mism, c = device_finish_pe(ix, mates, p)
+                n = res["n_cand"][0::2] + res["n_cand"][1::2]
+                assert (n > 48).sum() > 20 and (n > 100).any(), n.max()       # (fast mode: filter_pairs has already thinned the lists)
+                ofin, omism = ox.finish_pe(mates, res, cand, sensitive=bool(sensitive), ambiguous_out=bool(amb_out))
+                assert_same_pairs(fin, mism, ofin, omism)
+                if not amb_out:
+                    assert (fin["status"][0::2] == capi.FIN_AMBIGUOUS).sum() > 5, grid
+                else:
+                    assert (fin["flags"][0::2] & 2).astype(bool).sum() > 5, grid
+        finally:
+            ix.close()

@@ -21,13 +21,15 @@ ACGT = np.frombuffer(b"ACGT", dtype=np.uint8)
 # index residency variants (DESIGN.md §3): what the loader picks for a genome this small (dense suffix array, 16-mer table
 # only), the on-disk 1/8 suffix-array sampling with an 18-mer deep seed table, and the 20-mer table a 100 Mbp genome gets
 # and the layout of texts beyond 2^32 rows (bits 32..39 of every suffix-array value in their own byte array) forced onto
-# the small index together with the 20-mer table and the dense suffix array -- what a 3.1 Gbp genome gets
-@pytest.fixture(scope="module", params=["default", "sampled_sa+18mer", "20mer", "wide_sa+20mer"])
+# the small index together with the 20-mer table and the dense suffix array -- what a 3.1 Gbp genome gets; and the default
+# index with every persistent and grid-stride launch sized for one SM, so that each lane, warp and block of those kernels
+# takes many reads, windows and lists in turn (a batch of the suite is otherwise far smaller than one wave of their grids)
+@pytest.fixture(scope="module", params=["default", "sampled_sa+18mer", "20mer", "wide_sa+20mer", "small_grid"])
 def gidx(golden, request):
     import os
     env = {"default": {}, "sampled_sa+18mer": {"BMBS_SA": "sampled", "BMBS_KMER": "18"}, "20mer": {"BMBS_KMER": "20"},
-           "wide_sa+20mer": {"BMBS_FORCE_WIDE": "1", "BMBS_KMER": "20", "BMBS_SA": "dense"}}[request.param]
-    old = {k: os.environ.get(k) for k in ("BMBS_SA", "BMBS_KMER", "BMBS_FORCE_WIDE")}
+           "wide_sa+20mer": {"BMBS_FORCE_WIDE": "1", "BMBS_KMER": "20", "BMBS_SA": "dense"}, "small_grid": {"BMBS_GRID_SMS": "1"}}[request.param]
+    old = {k: os.environ.get(k) for k in ("BMBS_SA", "BMBS_KMER", "BMBS_FORCE_WIDE", "BMBS_GRID_SMS")}
     os.environ.update(env)
     try:
         ix = B.Index(golden / "genome.fa.index")
@@ -299,13 +301,15 @@ def test_verify_error_rate_other_than_default(gidx, oidx):
     ("pe100h", ["--seq1", "pe100h_1.fq", "--seq2", "pe100h_2.fq", "--pe"]),
     ("pe100hs", ["--seq1", "pe100h_1.fq", "--seq2", "pe100h_2.fq", "--pe", "--sensitive"]),
 ])
-@pytest.mark.parametrize("finish", ["device", "host", "device_warp_pairs"])
+@pytest.mark.parametrize("finish", ["device", "host", "device_warp_pairs", "device_small_grid"])
 def test_mapper_sam_identical_to_reference_golden(golden, built, name, args, finish):
     """whole program: FASTQ -> GPU seed-and-verify through the C ABI -> finishing (device: reduction / pair pick, ungapped CIGAR,
     coordinates, banded DP per launch; host: the same from the window lists) -> MAPQ -> SAM, vs the reference's SAM"""
     import os
-    # device_warp_pairs: every pair through the warp kernel of the pair finishing (staged lists, warp-parallel pair pick)
-    env = {**os.environ, **({"BMBS_HOST_FINISH": "1"} if finish == "host" else {"BMBS_PE_FIN_SHORT": "0"} if finish == "device_warp_pairs" else {})}
+    # device_warp_pairs: every pair through the warp kernel of the pair finishing (staged lists, warp-parallel pair pick);
+    # device_small_grid: every persistent and grid-stride launch sized for one SM, several batches in flight
+    env = {**os.environ, **{"host": {"BMBS_HOST_FINISH": "1"}, "device_warp_pairs": {"BMBS_PE_FIN_SHORT": "0"},
+                            "device_small_grid": {"BMBS_GRID_SMS": "1"}}.get(finish, {})}
     subprocess.run([str(built["bmbs"]), "--search", "genome.fa", *args, "-t", "4", "-o", "gpu.sam", "--mapstats", "gpu.stats", "--batch", "700"],
                    cwd=golden, check=True, stderr=subprocess.DEVNULL, env=env)
     assert sam_body(golden / "gpu.sam") == sam_body(golden / f"{name}.sam")

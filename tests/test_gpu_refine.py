@@ -16,9 +16,26 @@ from oracle_binding import OracleIndex, refine_final
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module")
-def gidx(golden):
-    ix = B.Index(golden / "genome.fa.index")
+# small_grid: refine_warp's grid sized for one SM (16 blocks of 4 warps), so that each warp takes many alignments in turn
+GRIDS = {"default": {}, "small_grid": {"BMBS_GRID_SMS": "1"}}
+
+
+def load_index(golden, env):
+    old = {k: os.environ.get(k) for k in env}
+    os.environ.update(env)
+    try:
+        return B.Index(golden / "genome.fa.index")
+    finally:
+        for k, v in old.items():
+            if v is None:
+                os.environ.pop(k, None)
+            else:
+                os.environ[k] = v
+
+
+@pytest.fixture(scope="module", params=list(GRIDS))
+def gidx(golden, request):
+    ix = load_index(golden, GRIDS[request.param])
     yield ix
     ix.close()
 
@@ -90,14 +107,17 @@ def test_refine_matches_cpu(gidx, oidx, seed, lengths, scoring, thread_kernel):
     rf.close()
 
 
-def test_refine_empty_and_reuse(gidx, oidx):
-    rf = B.Refiner(gidx)
-    res, ops = rf.refine(b"", b"", np.zeros(0, dtype=capi.RefineItem))
-    assert len(res) == 0 and len(ops) == 0
-    rng = np.random.default_rng(5)
-    for n in (3, 700, 40):                                     # buffers grow and are reused
-        seqs, quals, items = make_items(oidx, rng, n, [100], (6, 2, 1, 5, 3, 33))
-        res, ops = rf.refine(seqs, quals, items)
-        s0, qb0, qe0, nm0, c0 = refine_final(oidx, items[0]["site"], seqs[:100], quals[:100], int(items[0]["k"]))
-        assert (int(res[0]["score"]), int(res[0]["qb"]), int(res[0]["qe"]), int(res[0]["nm"])) == (s0, qb0, qe0, nm0)
-    rf.close()
+def test_refine_empty_and_reuse(golden, oidx):
+    for grid, env in GRIDS.items():
+        ix = load_index(golden, env)
+        rf = B.Refiner(ix)
+        res, ops = rf.refine(b"", b"", np.zeros(0, dtype=capi.RefineItem))
+        assert len(res) == 0 and len(ops) == 0
+        rng = np.random.default_rng(5)
+        for n in (3, 700, 40):                                     # buffers grow and are reused
+            seqs, quals, items = make_items(oidx, rng, n, [100], (6, 2, 1, 5, 3, 33))
+            res, ops = rf.refine(seqs, quals, items)
+            s0, qb0, qe0, nm0, c0 = refine_final(oidx, items[0]["site"], seqs[:100], quals[:100], int(items[0]["k"]))
+            assert (int(res[0]["score"]), int(res[0]["qb"]), int(res[0]["qe"]), int(res[0]["nm"])) == (s0, qb0, qe0, nm0), (grid, n)
+        rf.close()
+        ix.close()
