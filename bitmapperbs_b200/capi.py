@@ -245,7 +245,8 @@ class Batch:
         return nc.value, nm.value
 
     def finish(self):
-        """single end: reduction + ungapped CIGAR + coordinates on the device, behind run() on the batch's stream"""
+        """the finished records on the device, behind run() on the batch's stream: for single-end reads the reduction over the
+        window list, for pairs the hit compaction, distance filter and pair pick; then the ungapped CIGAR check and coordinates"""
         _check(self._L.bmbs_batch_finish(self._h))
 
     def download_final(self, fin=None, mism=None, cand=None):

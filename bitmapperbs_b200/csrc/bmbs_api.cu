@@ -401,6 +401,15 @@ extern "C" int bmbs_index_load(const char* index_prefix, const int* devices, int
 }
 
 // ================================================================================================ batch
+// what the host reads back after a run and a finish, copied into pinned memory on the batch's stream
+struct HostMirror {
+  u64 totals[2];                 // BatchView::totals[0..1]: candidate slots, verification work items
+  u32 status;                    // BatchView::status
+  u64 counters[8];               // BatchView::counters[0..7]
+  u64 out_cand;                  // BatchView::totals[3]: out_cand entries of all rounds
+  FinCounters fin;
+};
+
 struct bmbs_batch {
   bmbs_index* idx = nullptr; const DeviceCopy* copy = nullptr; int dev = 0;
   size_t max_reads = 0, max_bases = 0, cand_cap = 0;
@@ -409,18 +418,22 @@ struct bmbs_batch {
   BatchView v{};
   char* d_ascii = nullptr; u64* d_offsets = nullptr;
   u64* d_tile = nullptr;
-  u64* h_small = nullptr;        // pinned: totals[2], status, counters[8]; [16..23] finishing counters
+  HostMirror* mirror = nullptr;  // pinned
   cudaEvent_t ev[11] = {nullptr};
-  // finishing (bmbs_batch_finish): records, mismatch positions, handed-back window lists, reads to replay the sort for
-  bmbs_final* d_fin = nullptr; unsigned short* d_mism = nullptr; bmbs_cand* d_fb = nullptr; u32* d_sort_list = nullptr; u32* d_long_list = nullptr; u32* d_huge_list = nullptr; FinCounters* d_fc = nullptr;
-  size_t mism_cap = 0, fb_cap = 0; bool finished = false;
+  FinishView fv{};               // finishing (bmbs_batch_finish)
+  bool finished = false;
   int n_reads = 0, pe = 0, max_len = 0, launches = 0, sm_count = 148, seed_blocks_per_sm = 8; u32 seed_plane_cap = 0;
-  u32 pe_short = 48;             // pairs with more hits than this go to the warp kernel of the pair finishing (BMBS_PE_FIN_SHORT: tests)
   u32 seed_grid = 0, verify_grid = 0, verify_block = 0;   // as launched last (bmbs_batch_grid)
   bool ran = false;
 };
 
 namespace {
+// a finishing kernel over the batch's FinishView (FINISH_PARAMS)
+template <class K> void launch_finish(bmbs_batch* b, K kernel, u32 grid, u32 block, size_t smem) {
+  const FinishView& f = b->fv;
+  kernel<<<grid, block, smem, b->stream>>>(b->copy->view, b->v, f.fin, f.mism, f.mism_cap, f.fb, f.fb_cap, f.sort_list, f.long_list, f.huge_list, f.fc, f.pe_short);
+  ++b->launches;
+}
 // verify_windows over the work list.  Shared memory: five match planes of nch2 overlapping 64-bit chunks per thread; the 32-bit
 // band (every k <= 15) reads the chunk of its column only, the 64-bit band the one after it as well.  The grid is what is
 // resident at once (the kernel is a grid-stride loop over windows of equal cost: blocks beyond that would run alone at the end).
@@ -461,7 +474,7 @@ extern "C" void bmbs_batch_free(bmbs_batch* b) {
   if (!b) return;
   cudaSetDevice(b->dev);
   for (void* p : b->allocs) cudaFree(p);
-  if (b->h_small) cudaFreeHost(b->h_small);
+  if (b->mirror) cudaFreeHost(b->mirror);
   for (auto& e : b->ev) if (e) cudaEventDestroy(e);
   if (b->stream) cudaStreamDestroy(b->stream);
   delete b;
@@ -476,7 +489,6 @@ extern "C" int bmbs_batch_create(bmbs_index* idx, int dev, size_t max_reads, siz
   bmbs_batch* b = new bmbs_batch();
   b->idx = idx; b->copy = c; b->dev = dev; b->max_reads = max_reads; b->max_bases = max_bases; b->cand_cap = cand_cap;
   b->sm_count = c->grid_sms;
-  if (const char* e = getenv("BMBS_PE_FIN_SHORT")) b->pe_short = (u32)std::max(0, atoi(e));
   BatchView& v = b->v;
   const size_t R = max_reads + 2, S = cand_cap + 64;
   g_slab.clear();
@@ -496,10 +508,14 @@ extern "C" int bmbs_batch_create(bmbs_index* idx, int dev, size_t max_reads, siz
   A(dalloc(b, &v.scratch, (size_t)v.scratch_cap)); A(dalloc(b, &v.scratch_used, 4));
   A(dalloc(b, &v.counters, 16)); A(dalloc(b, &v.totals, 4)); A(dalloc(b, &v.status, 4));
   A(dalloc(b, &b->d_tile, R / SCAN_TILE + 8));
-  b->mism_cap = 32 * R;      // a read holds at most 31 mismatch positions b->fb_cap = S;
-  A(dalloc(b, &b->d_fin, R)); A(dalloc(b, &b->d_mism, b->mism_cap)); A(dalloc(b, &b->d_fb, b->fb_cap)); A(dalloc(b, &b->d_sort_list, R)); A(dalloc(b, &b->d_long_list, R)); A(dalloc(b, &b->d_huge_list, R)); A(dalloc(b, &b->d_fc, 1));
+  FinishView& f = b->fv;
+  f.mism_cap = (u32)(32 * R);          // a read holds at most 31 mismatch positions
+  f.fb_cap = (u32)S;                   // a handed-back read returns its whole slice of out_cand
+  A(dalloc(b, &f.fin, R)); A(dalloc(b, &f.mism, f.mism_cap)); A(dalloc(b, &f.fb, f.fb_cap)); A(dalloc(b, &f.sort_list, R)); A(dalloc(b, &f.long_list, R)); A(dalloc(b, &f.huge_list, R)); A(dalloc(b, &f.fc, 1));
+  f.pe_short = 48;                     // pairs with more hits go to finish_pe_long (BMBS_PE_FIN_SHORT: tests)
+  if (const char* e = getenv("BMBS_PE_FIN_SHORT")) f.pe_short = (u32)std::max(0, atoi(e));
   A(slab_commit(b));
-  A(cudaMallocHost((void**)&b->h_small, 48 * sizeof(u64)));
+  A(cudaMallocHost((void**)&b->mirror, sizeof(HostMirror)));
   for (auto& evt : b->ev) A(cudaEventCreate(&evt));
   if (e != cudaSuccess) { std::string m = std::string("batch allocation: ") + cudaGetErrorString(e); bmbs_batch_free(b); return fail(BMBS_ERR_CUDA, m); }
   v.slot_cap = cand_cap;
@@ -628,10 +644,11 @@ extern "C" int bmbs_batch_run(bmbs_batch* b, const bmbs_params* prm) {
     b->seed_grid = 0;
   }
   CU(cudaEventRecord(b->ev[8], s));
-  CU(cudaMemcpyAsync(b->h_small, v.totals, 2 * 8, cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(b->h_small + 12, v.totals + 3, 8, cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(b->h_small + 2, v.status, 4, cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(b->h_small + 4, v.counters, 8 * 8, cudaMemcpyDeviceToHost, s));
+  HostMirror* h = b->mirror;
+  CU(cudaMemcpyAsync(h->totals, v.totals, sizeof(h->totals), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&h->out_cand, v.totals + 3, sizeof(h->out_cand), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&h->status, v.status, sizeof(h->status), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(h->counters, v.counters, sizeof(h->counters), cudaMemcpyDeviceToHost, s));
   CU(cudaGetLastError());
   b->ran = true; b->finished = false;
   return BMBS_OK;
@@ -642,20 +659,21 @@ extern "C" int bmbs_batch_finish(bmbs_batch* b) {
   CU(cudaSetDevice(b->dev));
   cudaStream_t s = b->stream;
   const int n = b->n_reads;
-  CU(cudaMemsetAsync(b->d_fc, 0, sizeof(FinCounters), s));
+  const FinishView& f = b->fv;
+  CU(cudaMemsetAsync(f.fc, 0, sizeof(FinCounters), s));
   CU(cudaEventRecord(b->ev[9], s));
   if (n > 0 && b->pe) {
-    finish_pe<<<(n / 2 + 127) / 128, 128, 0, s>>>(b->copy->view, b->v, b->d_fin, b->d_mism, (u32)b->mism_cap, b->d_long_list, b->d_fc, b->pe_short); ++b->launches;
+    launch_finish(b, finish_pe, (n / 2 + 127) / 128, 128, 0);
     const size_t pe_smem = (size_t)PE_FIN_WARPS * 2 * PE_FIN_STAGE * sizeof(bmbs_cand);
-    finish_pe_long<<<b->sm_count * 2, 32 * PE_FIN_WARPS, pe_smem, s>>>(b->copy->view, b->v, b->d_fin, b->d_mism, (u32)b->mism_cap, b->d_long_list, b->d_fc); ++b->launches;
+    launch_finish(b, finish_pe_long, b->sm_count * 2, 32 * PE_FIN_WARPS, pe_smem);
   } else if (n > 0) {
-    finish_se<<<(n + 127) / 128, 128, 0, s>>>(b->copy->view, b->v, b->d_fin, b->d_mism, (u32)b->mism_cap, b->d_long_list, b->d_huge_list, b->d_sort_list, b->d_fc); ++b->launches;
-    finish_huge<<<b->sm_count * 2, 256, 0, s>>>(b->copy->view, b->v, b->d_fin, b->d_mism, (u32)b->mism_cap, b->d_fb, (u32)b->fb_cap, b->d_huge_list, b->d_sort_list, b->d_fc); ++b->launches;
-    finish_long<<<b->sm_count * 12, 128, 0, s>>>(b->copy->view, b->v, b->d_fin, b->d_mism, (u32)b->mism_cap, b->d_fb, (u32)b->fb_cap, b->d_long_list, b->d_sort_list, b->d_fc); ++b->launches;
-    finish_sorted<<<b->sm_count * 6, 32 * FIN_SORT_WARPS, 0, s>>>(b->copy->view, b->v, b->d_fin, b->d_mism, (u32)b->mism_cap, b->d_fb, (u32)b->fb_cap, b->d_sort_list, b->d_fc); ++b->launches;
+    launch_finish(b, finish_se, (n + 127) / 128, 128, 0);
+    launch_finish(b, finish_huge, b->sm_count * 2, 256, 0);
+    launch_finish(b, finish_long, b->sm_count * 12, 128, 0);
+    launch_finish(b, finish_sorted, b->sm_count * 6, 32 * FIN_SORT_WARPS, 0);
   }
   CU(cudaEventRecord(b->ev[10], s));
-  CU(cudaMemcpyAsync(b->h_small + 16, b->d_fc, sizeof(FinCounters), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(&b->mirror->fin, f.fc, sizeof(FinCounters), cudaMemcpyDeviceToHost, s));
   CU(cudaGetLastError());
   b->finished = true;
   return BMBS_OK;
@@ -670,10 +688,11 @@ extern "C" int bmbs_batch_sync(bmbs_batch* b) {
 
 namespace {
 int check_status(bmbs_batch* b, size_t* used) {
-  const u32 st = *(const u32*)(b->h_small + 2);
-  if (used) *used = (size_t)b->h_small[12];
+  const HostMirror& h = *b->mirror;
+  const u32 st = h.status;
+  if (used) *used = (size_t)h.out_cand;
   if (st & 1u) return fail(BMBS_ERR_CAPACITY, "a read produced more seed tasks than the per-read table holds");
-  if (st & 2u) { if (used) *used = (size_t)b->h_small[0]; return fail(BMBS_ERR_CAPACITY, "candidate slots exceed the batch capacity (" + std::to_string(b->h_small[0]) + " needed): create the batch with a larger cand_cap or send fewer reads"); }
+  if (st & 2u) { if (used) *used = (size_t)h.totals[0]; return fail(BMBS_ERR_CAPACITY, "candidate slots exceed the batch capacity (" + std::to_string(h.totals[0]) + " needed): create the batch with a larger cand_cap or send fewer reads"); }
   if (st & 4u) return fail(BMBS_ERR_CAPACITY, "verification work exceeds the batch capacity");
   if (st & 8u) return fail(BMBS_ERR_CAPACITY, "sort scratch exhausted");
   return BMBS_OK;
@@ -687,7 +706,7 @@ extern "C" int bmbs_batch_output_sizes(bmbs_batch* b, size_t* n_cand, size_t* n_
   if (n_mism) *n_mism = 0;
   int rc = check_status(b, n_cand);
   if (rc) return rc;
-  if (b->finished) { if (n_mism) *n_mism = (size_t)b->h_small[16]; if (n_cand) *n_cand = (size_t)b->h_small[17]; }
+  if (b->finished) { if (n_mism) *n_mism = (size_t)b->mirror->fin.mism_used; if (n_cand) *n_cand = (size_t)b->mirror->fin.fb_used; }
   return BMBS_OK;
 }
 
@@ -697,7 +716,7 @@ extern "C" int bmbs_batch_download(bmbs_batch* b, bmbs_read_result* res, bmbs_ca
   CU(cudaStreamSynchronize(b->stream));
   int rc = check_status(b, cand_used);
   if (rc) return rc;
-  const size_t work = (size_t)b->h_small[12];     // out_cand entries of all rounds
+  const size_t work = (size_t)b->mirror->out_cand;
   if (work > cand_cap) { if (cand_used) *cand_used = work; return fail(BMBS_ERR_CAPACITY, "caller's cand[] holds " + std::to_string(cand_cap) + " entries, " + std::to_string(work) + " needed"); }
   if (b->n_reads) CU(cudaMemcpyAsync(res, b->v.out_res, (size_t)b->n_reads * sizeof(bmbs_read_result), cudaMemcpyDeviceToHost, b->stream));
   if (work) { if (!cand) return fail(BMBS_ERR_ARG, "cand is null"); CU(cudaMemcpyAsync(cand, b->v.out_cand, work * sizeof(bmbs_cand), cudaMemcpyDeviceToHost, b->stream)); }
@@ -712,14 +731,15 @@ extern "C" int bmbs_batch_download_final(bmbs_batch* b, bmbs_final* fin, uint16_
   CU(cudaStreamSynchronize(b->stream));
   int rc = check_status(b, cand_used);
   if (rc) return rc;
-  const size_t nm = (size_t)b->h_small[16], nfb = (size_t)b->h_small[17];
+  const FinishView& f = b->fv;
+  const size_t nm = (size_t)b->mirror->fin.mism_used, nfb = (size_t)b->mirror->fin.fb_used;
   if (mism_used) *mism_used = nm;
   if (cand_used) *cand_used = nfb;
-  if (nm > b->mism_cap || nfb > b->fb_cap) return fail(BMBS_ERR_CAPACITY, "finishing buffers of the batch are too small");
+  if (nm > f.mism_cap || nfb > f.fb_cap) return fail(BMBS_ERR_CAPACITY, "finishing buffers of the batch are too small");
   if (nm > mism_cap || nfb > cand_cap) return fail(BMBS_ERR_CAPACITY, "caller's mism[] / cand[] too small: " + std::to_string(nm) + " / " + std::to_string(nfb) + " entries needed");
-  if (b->n_reads) CU(cudaMemcpyAsync(fin, b->d_fin, (size_t)b->n_reads * sizeof(bmbs_final), cudaMemcpyDeviceToHost, b->stream));
-  if (nm) { if (!mism) return fail(BMBS_ERR_ARG, "mism is null"); CU(cudaMemcpyAsync(mism, b->d_mism, nm * sizeof(uint16_t), cudaMemcpyDeviceToHost, b->stream)); }
-  if (nfb) { if (!cand) return fail(BMBS_ERR_ARG, "cand is null"); CU(cudaMemcpyAsync(cand, b->d_fb, nfb * sizeof(bmbs_cand), cudaMemcpyDeviceToHost, b->stream)); }
+  if (b->n_reads) CU(cudaMemcpyAsync(fin, f.fin, (size_t)b->n_reads * sizeof(bmbs_final), cudaMemcpyDeviceToHost, b->stream));
+  if (nm) { if (!mism) return fail(BMBS_ERR_ARG, "mism is null"); CU(cudaMemcpyAsync(mism, f.mism, nm * sizeof(uint16_t), cudaMemcpyDeviceToHost, b->stream)); }
+  if (nfb) { if (!cand) return fail(BMBS_ERR_ARG, "cand is null"); CU(cudaMemcpyAsync(cand, f.fb, nfb * sizeof(bmbs_cand), cudaMemcpyDeviceToHost, b->stream)); }
   CU(cudaStreamSynchronize(b->stream));
   return BMBS_OK;
 }
@@ -728,7 +748,8 @@ extern "C" int bmbs_batch_finish_counters(bmbs_batch* b, uint64_t c[8]) {
   if (!b || !b->finished || !c) return fail(BMBS_ERR_ARG, "bad argument or batch not finished");
   CU(cudaSetDevice(b->dev));
   CU(cudaStreamSynchronize(b->stream));
-  for (int i = 0; i < 8; ++i) c[i] = b->h_small[16 + i];
+  const FinCounters& f = b->mirror->fin;
+  c[0] = f.mism_used; c[1] = f.fb_used; c[2] = f.n_sorted; c[3] = f.n_host; c[4] = f.n_dp; c[5] = f.n_unc_idx; c[6] = f.n_unc_sbd;
   float ms = 0; CU(cudaEventElapsedTime(&ms, b->ev[9], b->ev[10]));
   c[7] = (uint64_t)(ms * 1000.0f);
   return BMBS_OK;
@@ -747,8 +768,8 @@ extern "C" int bmbs_batch_counters(bmbs_batch* b, uint64_t c[8]) {
   if (!b || !b->ran || !c) return fail(BMBS_ERR_ARG, "bad argument or batch not run");
   CU(cudaSetDevice(b->dev));
   CU(cudaStreamSynchronize(b->stream));
-  for (int i = 0; i < 8; ++i) c[i] = b->h_small[4 + i];
-  c[CNT_CAND] = b->h_small[0];
+  for (int i = 0; i < 8; ++i) c[i] = b->mirror->counters[i];
+  c[CNT_CAND] = b->mirror->totals[0];
   return BMBS_OK;
 }
 
@@ -823,7 +844,7 @@ int map_batch(bmbs_index* idx, int dev, const char* seqs, const uint64_t* offset
     if ((rc = bmbs_batch_upload(b, seqs, offsets, n_reads, pe))) return rc;
     if ((rc = bmbs_batch_run(b, prm))) return rc;
     rc = bmbs_batch_download(b, res, cand, cand_cap, cand_used);
-    if (rc == BMBS_ERR_CAPACITY && (*(const u32*)(b->h_small + 2) & 2u)) { dev_cap = (size_t)b->h_small[0] + (size_t)(b->h_small[0] >> 2) + 1024; continue; }
+    if (rc == BMBS_ERR_CAPACITY && (b->mirror->status & 2u)) { const size_t slots = (size_t)b->mirror->totals[0]; dev_cap = slots + (slots >> 2) + 1024; continue; }
     return rc;
   }
   return fail(BMBS_ERR_CAPACITY, "candidate slots keep exceeding the device capacity");
@@ -878,9 +899,10 @@ extern "C" int bmbs_batch_verify(bmbs_batch* b, const uint32_t* read_idx, const 
   for (int i = 1; i <= 5; ++i) CU(cudaEventRecord(b->ev[i], s));
   launch_verify(b, v.e_rate, s, b->copy->view, v);
   CU(cudaEventRecord(b->ev[6], s)); CU(cudaEventRecord(b->ev[7], s)); CU(cudaEventRecord(b->ev[8], s));
-  CU(cudaMemcpyAsync(b->h_small + 4, v.counters, 8 * 8, cudaMemcpyDeviceToHost, s));
+  HostMirror* h = b->mirror;
+  CU(cudaMemcpyAsync(h->counters, v.counters, sizeof(h->counters), cudaMemcpyDeviceToHost, s));
   CU(cudaGetLastError());
-  b->h_small[0] = 0; b->h_small[1] = n; b->h_small[12] = n; *(u32*)(b->h_small + 2) = 0; b->ran = true;
+  h->totals[0] = 0; h->totals[1] = n; h->out_cand = n; h->status = 0; b->ran = true;
   return BMBS_OK;
 }
 
