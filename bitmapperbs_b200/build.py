@@ -34,7 +34,7 @@ def _run(cmd):
 
 
 def build_library(force=False) -> Path:
-    src = [PKG / "csrc/bmbs_api.cu", PKG / "csrc/bmbs_kernels.cuh", PKG / "csrc/bmbs_device.cuh", PKG / "csrc/bmbs_sort_replay.h", PKG / "csrc/bmbs_band_walk.h", PKG / "csrc/bmbs_finish_pe.cuh", ROOT / "include/bmbs.h"]
+    src = [PKG / "csrc/bmbs_api.cu", PKG / "csrc/bmbs_kernels.cuh", PKG / "csrc/bmbs_device.cuh", PKG / "csrc/bmbs_sort_replay.h", PKG / "csrc/bmbs_band_walk.h", PKG / "csrc/bmbs_refine_ends.h", PKG / "csrc/bmbs_finish_pe.cuh", ROOT / "include/bmbs.h"]
     if force or _newer(LIB, src):
         _run([NVCC, *NVCC_FLAGS, "-shared", src[0], "-o", LIB])
     return LIB
@@ -42,7 +42,7 @@ def build_library(force=False) -> Path:
 
 def build_tools(force=False):
     OUT.mkdir(exist_ok=True)
-    host = sorted((PKG / "csrc/host").glob("*.hpp")) + sorted((PKG / "indexer").glob("*.hpp"))
+    host = sorted((PKG / "csrc/host").glob("*.hpp")) + sorted((PKG / "indexer").glob("*.hpp")) + [PKG / "csrc/bmbs_refine_ends.h"]
     idx = OUT / "bmbs-index"
     if force or _newer(idx, [PKG / "indexer/build_index.cpp", *host]):
         _run(["g++", "-O2", "-std=c++17", "-pthread", PKG / "indexer/build_index.cpp", "-o", idx])

@@ -940,8 +940,7 @@ struct bmbs_refiner {
   cudaStream_t stream = nullptr;
   // device buffers, grown on demand
   char* d_seq = nullptr; char* d_qual = nullptr; size_t cap_bytes = 0;
-  bmbs_refine_item* d_items = nullptr; bmbs_refine_result* d_res = nullptr; u64* d_dir_off = nullptr; u64* d_ops_off = nullptr; size_t cap_items = 0;
-  unsigned char* d_dir = nullptr; size_t cap_dir = 0;
+  bmbs_refine_item* d_items = nullptr; bmbs_refine_result* d_res = nullptr; u64* d_ops_off = nullptr; size_t cap_items = 0;
   u32* d_ops_scratch = nullptr; u32* d_ops_out = nullptr; size_t cap_ops = 0;
   unsigned long long* d_total = nullptr;
   // page-locked staging for the offsets and the counter
@@ -960,7 +959,8 @@ extern "C" int bmbs_refiner_create(bmbs_index* idx, int dev, bmbs_refiner** out)
   r->idx = idx; r->copy = copy; r->dev = dev;
   CU(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking));
   r->sm_count = copy->grid_sms;
-  cudaFuncSetAttribute(refine_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, RW_WARPS * 1000 * (int)sizeof(uint4));
+  cudaFuncSetAttribute(refine_warp<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, RW_WARPS * 1000 * (int)sizeof(uint4));
+  cudaFuncSetAttribute(refine_warp<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, RW_WARPS * 1000 * 2 * (int)sizeof(uint4));
   CU(cudaMalloc(&r->d_total, 8));
   CU(cudaMallocHost(&r->h_total, 8));
   CU(cudaEventCreate(&r->ev0)); CU(cudaEventCreate(&r->ev1));
@@ -972,8 +972,8 @@ extern "C" void bmbs_refiner_free(bmbs_refiner* r) {
   if (!r) return;
   cudaSetDevice(r->dev);
   cudaStreamSynchronize(r->stream);
-  cudaFree(r->d_seq); cudaFree(r->d_qual); cudaFree(r->d_items); cudaFree(r->d_res); cudaFree(r->d_dir_off); cudaFree(r->d_ops_off);
-  cudaFree(r->d_dir); cudaFree(r->d_ops_scratch); cudaFree(r->d_ops_out); cudaFree(r->d_total);
+  cudaFree(r->d_seq); cudaFree(r->d_qual); cudaFree(r->d_items); cudaFree(r->d_res); cudaFree(r->d_ops_off);
+  cudaFree(r->d_ops_scratch); cudaFree(r->d_ops_out); cudaFree(r->d_total);
   cudaFreeHost(r->h_off); cudaFreeHost(r->h_total);
   if (r->ev0) cudaEventDestroy(r->ev0); if (r->ev1) cudaEventDestroy(r->ev1);
   cudaStreamDestroy(r->stream);
@@ -986,39 +986,31 @@ extern "C" int bmbs_refine(bmbs_refiner* r, const char* seqs, const char* quals,
   if (ops_used) *ops_used = 0;
   if (n == 0) return BMBS_OK;
   CU(cudaSetDevice(r->dev));
-  // per-item scratch: band x L direction bytes and 2L + 2k + 2 ops (the longest possible traceback)
-  if (2 * (n + 1) > r->cap_h_off) { cudaFreeHost(r->h_off); r->cap_h_off = 2 * (n + 1) + 1024; CU(cudaMallocHost(&r->h_off, r->cap_h_off * 8)); }
-  u64* dir_off = r->h_off; u64* ops_off = r->h_off + (n + 1);
-  u64 dir_total = 0, ops_total = 0;
-  // bands of up to 32 cells go to the warp kernel (directions in shared memory), wider ones to the thread kernel
-  const int all_thread = getenv("BMBS_REFINE_THREAD") ? 1 : 0;      // tests: every item through the thread kernel
-  size_t n_warp = 0, n_thread = 0; u32 max_len = 1;
+  // per-item scratch: 2L + 2k + 2 ops (the longest possible traceback)
+  if (n + 1 > r->cap_h_off) { cudaFreeHost(r->h_off); r->cap_h_off = n + 1 + 1024; CU(cudaMallocHost(&r->h_off, r->cap_h_off * 8)); }
+  u64* ops_off = r->h_off;
+  u64 ops_total = 0;
+  // bands of up to 32 cells go to refine_warp<1>, wider ones (up to 63) to refine_warp<2>
+  size_t n_cls[2] = {0, 0}; u32 max_len[2] = {1, 1};
   for (size_t i = 0; i < n; ++i) {
     const bmbs_refine_item& q = items[i];
     if (q.k > 31) return fail(BMBS_ERR_ARG, "k > 31");
     if (q.len == 0 || q.len > 1000) return fail(BMBS_ERR_ARG, "read length outside 1..1000");
     if ((size_t)q.seq_off + q.len > bytes) return fail(BMBS_ERR_ARG, "item reaches past the end of seqs[]");
-    const bool warp_item = !all_thread && 2 * q.k + 1 <= 32;
-    if (warp_item) { ++n_warp; if (q.len > max_len) max_len = q.len; } else ++n_thread;
-    dir_off[i] = dir_total; ops_off[i] = ops_total;
-    if (!warp_item) dir_total += (u64)(2 * q.k + 1) * q.len;
+    const int c = 2 * q.k + 1 > 32;
+    ++n_cls[c]; if (q.len > max_len[c]) max_len[c] = q.len;
+    ops_off[i] = ops_total;
     ops_total += 2ull * q.len + 2ull * q.k + 2;
   }
-  dir_off[n] = dir_total; ops_off[n] = ops_total;
+  ops_off[n] = ops_total;
   if (ops_total > 0xFFFFFFFFull) return fail(BMBS_ERR_CAPACITY, "too many alignments in one bmbs_refine call");
-  auto grow = [&](void** p, size_t& cap, size_t need, size_t elem) -> cudaError_t {
-    if (need <= cap) return cudaSuccess;
-    cudaFree(*p); *p = nullptr; cap = need + need / 2 + 1024;
-    return cudaMalloc(p, cap * elem);
-  };
   if (bytes > r->cap_bytes) { cudaFree(r->d_seq); cudaFree(r->d_qual); r->d_seq = r->d_qual = nullptr; r->cap_bytes = bytes + bytes / 2 + 4096; CU(cudaMalloc(&r->d_seq, r->cap_bytes)); CU(cudaMalloc(&r->d_qual, r->cap_bytes)); }
   if (n + 1 > r->cap_items) {
-    cudaFree(r->d_items); cudaFree(r->d_res); cudaFree(r->d_dir_off); cudaFree(r->d_ops_off);
+    cudaFree(r->d_items); cudaFree(r->d_res); cudaFree(r->d_ops_off);
     r->cap_items = n + n / 2 + 1024;
     CU(cudaMalloc(&r->d_items, r->cap_items * sizeof(bmbs_refine_item))); CU(cudaMalloc(&r->d_res, r->cap_items * sizeof(bmbs_refine_result)));
-    CU(cudaMalloc(&r->d_dir_off, r->cap_items * 8)); CU(cudaMalloc(&r->d_ops_off, r->cap_items * 8));
+    CU(cudaMalloc(&r->d_ops_off, r->cap_items * 8));
   }
-  CU(grow((void**)&r->d_dir, r->cap_dir, (size_t)dir_total + 64, 1));
   if (ops_total > r->cap_ops) {
     cudaFree(r->d_ops_scratch); cudaFree(r->d_ops_out); r->d_ops_scratch = r->d_ops_out = nullptr;
     r->cap_ops = (size_t)ops_total + (size_t)ops_total / 2 + 1024;
@@ -1028,20 +1020,17 @@ extern "C" int bmbs_refine(bmbs_refiner* r, const char* seqs, const char* quals,
   CU(cudaMemcpyAsync(r->d_seq, seqs, bytes, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(r->d_qual, quals, bytes, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(r->d_items, items, n * sizeof(bmbs_refine_item), cudaMemcpyHostToDevice, s));
-  CU(cudaMemcpyAsync(r->d_dir_off, dir_off, (n + 1) * 8, cudaMemcpyHostToDevice, s));
   CU(cudaMemcpyAsync(r->d_ops_off, ops_off, (n + 1) * 8, cudaMemcpyHostToDevice, s));
   CU(cudaMemsetAsync(r->d_total, 0, 8, s));
   RefineScoring rs{sc->mp_max, sc->mp_min, sc->n_pen, sc->gap_open, sc->gap_ext, sc->q_base};
   CU(cudaEventRecord(r->ev0, s));
-  if (n_warp) {
-    const size_t smem = (size_t)RW_WARPS * max_len * sizeof(uint4);
-    const unsigned blocks = (unsigned)std::min<size_t>((n + RW_WARPS - 1) / RW_WARPS, (size_t)r->sm_count * 16);
-    refine_warp<<<blocks, 32 * RW_WARPS, smem, s>>>(r->copy->view, r->d_items, (u32)n, r->d_seq, r->d_qual, rs, r->d_ops_scratch, r->d_ops_off, r->d_res,
-                                                   r->d_ops_out, r->d_total, (u64)r->cap_ops, max_len);
+  for (int c = 0; c < 2; ++c) {
+    if (!n_cls[c]) continue;
+    const size_t smem = (size_t)RW_WARPS * max_len[c] * (c + 1) * sizeof(uint4);
+    const unsigned blocks = (unsigned)std::min<size_t>((n_cls[c] + RW_WARPS - 1) / RW_WARPS, (size_t)r->sm_count * 16);
+    (c ? refine_warp<2> : refine_warp<1>)<<<blocks, 32 * RW_WARPS, smem, s>>>(r->copy->view, r->d_items, (u32)n, r->d_seq, r->d_qual, rs, r->d_ops_scratch,
+                                                                             r->d_ops_off, r->d_res, r->d_ops_out, r->d_total, (u64)r->cap_ops, max_len[c]);
   }
-  if (n_thread)
-    refine_dp<<<(unsigned)((n + 63) / 64), 64, 0, s>>>(r->copy->view, r->d_items, (u32)n, r->d_seq, r->d_qual, rs, r->d_dir, r->d_dir_off,
-                                                        r->d_ops_scratch, r->d_ops_off, r->d_res, r->d_ops_out, r->d_total, (u64)r->cap_ops, all_thread);
   CU(cudaEventRecord(r->ev1, s)); r->timed = true;
   CU(cudaMemcpyAsync(r->h_total, r->d_total, 8, cudaMemcpyDeviceToHost, s));
   CU(cudaMemcpyAsync(res, r->d_res, n * sizeof(bmbs_refine_result), cudaMemcpyDeviceToHost, s));

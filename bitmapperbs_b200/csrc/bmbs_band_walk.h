@@ -12,10 +12,12 @@
 #pragma once
 #include <cstdint>
 
+#ifndef BMBS_HD
 #if defined(__CUDACC__)
 #define BMBS_HD __host__ __device__ __forceinline__
 #else
 #define BMBS_HD inline
+#endif
 #endif
 
 namespace bmbs {

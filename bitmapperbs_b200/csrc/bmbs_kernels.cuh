@@ -11,7 +11,8 @@
 //   gather_work      the surviving windows as one VerifyItem each (resolved reads get their record directly)
 //   verify_windows   kernel 3: banded Myers bit-vector edit distance, read T may face reference C
 //   sens_pair, reseed_clear, seed_reseed, sens_reseed_filter, sens_reseed_finish   --pe --sensitive: pair logic and the re-seeding round
-//   refine_dp, refine_warp   CIGAR refinement: banded affine-gap DP with traceback (SURVEY 8f-1), a thread / a warp per item
+//   refine_warp<1>, refine_warp<2>   CIGAR refinement: banded affine-gap DP with traceback (SURVEY 8f-1), a warp per item,
+//                    one or two band cells per lane
 //   finalize_reads   per-read result records
 //   finish_se, finish_long, finish_huge, finish_sorted   single-end finishing on the device: a thread / a warp / a CTA per
 //                    read by the length of its window list, and the replay of std::sort's order where the order decides
@@ -22,6 +23,7 @@
 #include "bmbs_device.cuh"
 #include "bmbs_sort_replay.h"
 #include "bmbs_band_walk.h"
+#include "bmbs_refine_ends.h"
 #include "../../include/bmbs.h"
 
 namespace bmbs {
@@ -1407,37 +1409,15 @@ __global__ void __launch_bounds__(128, 7) verify_windows(DevIndex ix, BatchView 
 // semi-global banded (2k+1) affine-gap alignment of the read against its window with traceback, then the end fix-ups
 // (leading / trailing insertions become matches, :2894-2990) and the NM recount over the final operations (:2990-3143).
 // Values and tie-breaks are the reference's, cell by cell (every comparison below is written as it is there).
-//   refine_warp   bands of up to 32 cells (k <= 15): one warp per alignment, one band cell per lane.  Within a row the match
-//                 score m and the vertical gap e only depend on the row above (m: the lane's own h, e: the neighbour lane's),
-//                 and the horizontal gap opens from m alone, f[j+1] = max(f[j] - ext, m[j] - open - ext): a max-plus prefix
-//                 scan over the lanes.  The four direction bits of a row are four ballots, kept in shared memory (16 bytes
-//                 per row), so the DP touches global memory only for the read, its qualities and the window.
-//   refine_dp     wider bands (k 16..31): one thread per alignment, H / E rows in a 128-entry ring, direction bytes in global
-//                 scratch.
+//   refine_warp<C>   one warp per alignment, C band cells per lane: lane l holds cells l and l + 32 (C = 1 for bands of up to
+//                    32 cells, k <= 15; C = 2 for up to 63 cells, k 16..31).  Within a row the match score m and the vertical
+//                    gap e only depend on the row above (m: the cell's own h, e: the next cell's), and the horizontal gap opens
+//                    from m alone, f[j+1] = max(f[j] - ext, m[j] - open - ext): a max-plus prefix scan over the lanes, one
+//                    half after the other.  The four direction bits of a row are four ballots per half, kept in shared memory
+//                    (C x 16 bytes per row), so the DP touches global memory only for the read, its qualities and the window.
+//                    The end fix-ups are refine_fix_ends (bmbs_refine_ends.h), the same code the CPU refinement runs.
 struct RefineScoring { int mp_max, mp_min, n_pen, gap_open, gap_ext, q_base; };
 
-// End fix-ups of the traceback in ops[0..n) (read order, (len << 4) | op, 0 = M, 1 = D, 2 = I): the read is aligned end to end,
-// so insertions at either end become matches and the window span grows with them.  Returns the first / last op that stays.
-__device__ __forceinline__ void refine_fix_ends(u32* ops, int n, int& qb, int& qe, int& cb, int& ce) {
-  int i = 0; u32 ins = 0;
-  for (; i < n && (ops[i] & 0xfu) == 2u; ++i) ins += ops[i] >> 4;
-  if (i != 0) {
-    u32 op = ops[i] & 0xfu, len = ops[i] >> 4;
-    if (op == 0) len += ins; else { op = 0; len = ins; --i; }
-    ops[i] = len << 4 | op;
-    qb -= (int)ins;
-  }
-  cb = i;
-  ins = 0;
-  for (i = n - 1; i >= cb && (ops[i] & 0xfu) == 2u; --i) ins += ops[i] >> 4;
-  if (i != n - 1) {
-    u32 op = ops[i] & 0xfu, len = ops[i] >> 4;
-    if (op == 0) len += ins; else { op = 0; len = ins; ++i; }
-    ops[i] = len << 4 | op;
-    qe += (int)ins;
-  }
-  ce = i;
-}
 // read character against the window base at double-strand position pos (an out-of-strand window matches nothing)
 __device__ __forceinline__ u32 refine_mismatch(const DevIndex& ix, bool inside, u64 pos, char rc) {
   if (!inside) return 1u;
@@ -1449,131 +1429,33 @@ __device__ __forceinline__ int refine_nt4(char c) {
   switch (c) { case 'A': case 'a': return 0; case 'C': case 'c': return 1; case 'G': case 'g': return 2; case 'T': case 't': return 3; default: return 4; }
 }
 
-__global__ void __launch_bounds__(64) refine_dp(DevIndex ix, const bmbs_refine_item* __restrict__ items, u32 n, const char* __restrict__ seqs,
-                                                const char* __restrict__ quals, RefineScoring sc, unsigned char* __restrict__ dir_all,
-                                                const u64* __restrict__ dir_off, u32* __restrict__ ops_scratch, const u64* __restrict__ ops_off,
-                                                bmbs_refine_result* __restrict__ res, u32* __restrict__ ops_out, unsigned long long* ops_total, u64 ops_cap, int all_items) {
-  const u32 it = blockIdx.x * blockDim.x + threadIdx.x;
-  if (it >= n) return;
-  const bmbs_refine_item q = items[it];
-  if (2 * (int)q.k + 1 <= 32 && !all_items) return;      // refine_warp's
-  const int rlen = q.len, k = q.k, band = 2 * k + 1, wlen = rlen + 2 * k;
-  const char* read = seqs + q.seq_off; const char* qual = quals + q.seq_off;
-  const int NEG = -0x40000000, goe = sc.gap_open + sc.gap_ext, ge = sc.gap_ext;
-  const bool inside = window_inside(ix, q.site, (u64)wlen);
-  int H[128], E[128];                                  // ring over window positions: row i touches j in [i, i + band], band <= 63
-  for (int j = 0; j < 128; ++j) { H[j] = NEG; E[j] = NEG; }
-  for (int j = 0; j < band; ++j) { H[j] = 0; E[j] = -goe; }
-  unsigned char* dir = dir_all + dir_off[it];
-  const uint2* gp = ix.planes + (q.site >> 5);
-  const unsigned sh0 = (unsigned)q.site & 31u;
-  int beg = 0, end = 0;
-  for (int i = 0; i < rlen; ++i) {
-    const int t = refine_nt4(read[i]);
-    double phred = (double)((int)qual[i] - sc.q_base);
-    if (phred > 40) phred = 40;
-    phred = phred / 40;
-    const int mism = -sc.mp_min - (int)((double)(signed char)(sc.mp_max - sc.mp_min) * phred);
-    beg = i; end = i + band;
-    // window bases [i, i + 64) as two 64-bit planes (code = lo | hi << 1: A0 C1 G2 T3)
-    u64 wlo = 0, whi = 0;
-    if (inside) {
-      const unsigned bit = sh0 + (unsigned)i;
-      const uint2* wp = gp + (bit >> 5); const unsigned s = bit & 31u;
-      const uint2 a = __ldg(wp), b2 = __ldg(wp + 1), c = __ldg(wp + 2);
-      wlo = (u64)__funnelshift_r(a.x, b2.x, s) | ((u64)__funnelshift_r(b2.x, c.x, s) << 32);
-      whi = (u64)__funnelshift_r(a.y, b2.y, s) | ((u64)__funnelshift_r(b2.y, c.y, s) << 32);
-    }
-    int f = NEG, left = NEG;
-    unsigned char* d_row = dir + (size_t)i * band;
-    for (int j = beg; j < end; ++j) {
-      const int jj = j - beg;
-      int m = H[j & 127], e = E[j & 127];
-      H[j & 127] = left;
-      const int qb = inside ? (int)(((wlo >> jj) & 1ull) | (((whi >> jj) & 1ull) << 1)) : 4;
-      int s;
-      if (t == 4 || qb == 4) s = -sc.n_pen;
-      else if (t == qb || (t == 3 && qb == 1)) s = 0;
-      else s = mism;
-      m += s;
-      unsigned char d = m >= e ? 0 : 1;
-      int h = m >= e ? m : e;
-      d = h >= f ? d : 2;
-      h = h >= f ? h : f;
-      left = h;
-      const int open = m - goe;
-      e -= ge;
-      if (e > open) d |= 1 << 2; else e = open;
-      E[j & 127] = e;
-      f -= ge;
-      if (f > open) d |= 2 << 4; else f = open;
-      d_row[jj] = d;
-    }
-    H[end & 127] = left; E[end & 127] = NEG;
-  }
-  int best = rlen + k;
-  int score = H[best & 127];
-  for (int j = end; j > beg; --j) if (H[j & 127] > score) { score = H[j & 127]; best = j; }
-  // traceback, ops pushed from the alignment end; written backwards so that they read in read order
-  u32* ops = ops_scratch + ops_off[it];
-  const u32 cap = (u32)(ops_off[it + 1] - ops_off[it]);
-  u32 n_ops = 0, cur = 0;                               // cur: the run being built, (len << 4) | op
-  auto push = [&](u32 op, u32 len) {
-    if (n_ops == 0 || (cur & 0xfu) != op) { if (n_ops) ops[cap - n_ops] = cur; cur = len << 4 | op; ++n_ops; } else cur += len << 4;
-  };
-  int i = rlen - 1, j = best - 1, state = 0;
-  while (i >= 0 && j >= 0) {
-    state = dir[(size_t)i * band + (j - i)] >> (state << 1) & 3;
-    if (state == 0) { push(0, 1); --i; --j; }
-    else if (state == 1) { push(2, 1); --i; }
-    else { push(1, 1); --j; }
-  }
-  if (i >= 0) push(2, (u32)(i + 1));
-  if (n_ops) ops[cap - n_ops] = cur;
-  int qb = j + 1, qe = best - 1, cb = 0, ce = -1;
-  u32* fo = ops + (cap - n_ops);
-  if (n_ops) refine_fix_ends(fo, (int)n_ops, qb, qe, cb, ce);
-  u32 nm = 0;
-  {
-    int wi = qb, ri = 0;
-    for (int x = cb; x <= ce; ++x) {
-      const u32 op = fo[x] & 0xfu, len = fo[x] >> 4;
-      if (op == 0) { for (u32 y = 0; y < len; ++y) nm += refine_mismatch(ix, inside, q.site + (u64)(long long)(wi + (int)y), read[ri + (int)y]); wi += (int)len; ri += (int)len; }
-      else if (op == 1) { wi += (int)len; nm += len; }
-      else { ri += (int)len; nm += len; }
-    }
-  }
-  const u32 n_fin = ce >= cb ? (u32)(ce - cb + 1) : 0u;
-  const u64 at = atomicAdd(ops_total, (unsigned long long)n_fin);
-  if (at + n_fin <= ops_cap) for (u32 x = 0; x < n_fin; ++x) ops_out[at + x] = fo[cb + (int)x];
-  bmbs_refine_result r; r.score = score; r.qb = qb; r.qe = qe; r.n_ops = n_fin; r.ops_off = (u32)at; r.nm = nm;
-  res[it] = r;
-}
-
 constexpr int RW_WARPS = 4;
+template <int C>
 __global__ void __launch_bounds__(32 * RW_WARPS) refine_warp(DevIndex ix, const bmbs_refine_item* __restrict__ items, u32 n, const char* __restrict__ seqs,
                                                              const char* __restrict__ quals, RefineScoring sc, u32* __restrict__ ops_scratch, const u64* __restrict__ ops_off,
                                                              bmbs_refine_result* __restrict__ res, u32* __restrict__ ops_out, unsigned long long* ops_total, u64 ops_cap, u32 max_len) {
-  extern __shared__ uint4 s_dirs[];                     // [RW_WARPS][max_len]: bit jj of .x/.y = h source, .z = e extended, .w = f extended
+  // [RW_WARPS][max_len][C]: bit l of .x/.y = h source of cell l + 32c, .z = e extended, .w = f extended
+  extern __shared__ uint4 s_dirs[];
   __shared__ int s_fin[RW_WARPS][8];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  uint4* dir = s_dirs + (size_t)w * max_len;
+  uint4* dir = s_dirs + (size_t)w * max_len * C;
   const u32 warps = gridDim.x * RW_WARPS;
   const int NEG = -0x40000000, goe = sc.gap_open + sc.gap_ext, ge = sc.gap_ext;
   for (u32 it = blockIdx.x * RW_WARPS + w; it < n; it += warps) {
     const bmbs_refine_item q = items[it];
     const int rlen = q.len, k = q.k, band = 2 * k + 1, wlen = rlen + 2 * k;
-    if (band > 32) continue;                            // refine_dp's
+    if ((band > 32) != (C > 1)) continue;               // the other instance's
     const char* read = seqs + q.seq_off; const char* qual = quals + q.seq_off;
     const bool inside = window_inside(ix, q.site, (u64)wlen);
-    const bool act = lane < band;
-    int hd = 0, e_prev = -goe;                          // row 0: H = 0, E = -(open + ext) over the band
-    int my_t = 4, my_mism = 0; u32 wlo = 0, whi = 0;
+    bool act[C]; int hd[C], e_prev[C]; u32 wlo[C], whi[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) { act[c] = lane + 32 * c < band; hd[c] = 0; e_prev[c] = -goe; wlo[c] = whi[c] = 0; }   // row 0: H = 0, E = -(open + ext)
+    int my_t = 4, my_mism = 0;
     for (int i = 0; i < rlen; ++i) {
       const int ph = i & 31;
       if (ph == 0) {
-        // every 32 rows: lane l prepares row i + l (base code, quality-scaled mismatch penalty) and its own diagonal's next
-        // 32 window bases (window position i + lane + 0..31)
+        // every 32 rows: lane l prepares row i + l (base code, quality-scaled mismatch penalty) and the next 32 window bases of
+        // each of its diagonals (window position i + lane + 32c + 0..31)
         const int ri = i + lane;
         my_t = 4; my_mism = 0;
         if (ri < rlen) {
@@ -1584,46 +1466,64 @@ __global__ void __launch_bounds__(32 * RW_WARPS) refine_warp(DevIndex ix, const 
           my_mism = -sc.mp_min - (int)((double)(signed char)(sc.mp_max - sc.mp_min) * phred);
         }
         if (inside) {
-          const u64 p = q.site + (u64)(i + lane);
-          const uint2 g0 = __ldg(ix.planes + (p >> 5)), g1 = __ldg(ix.planes + (p >> 5) + 1);
-          const unsigned sh = (unsigned)p & 31u;
-          wlo = __funnelshift_r(g0.x, g1.x, sh); whi = __funnelshift_r(g0.y, g1.y, sh);
+#pragma unroll
+          for (int c = 0; c < C; ++c) {
+            const u64 p = q.site + (u64)(i + lane + 32 * c);
+            const uint2 g0 = __ldg(ix.planes + (p >> 5)), g1 = __ldg(ix.planes + (p >> 5) + 1);
+            const unsigned sh = (unsigned)p & 31u;
+            wlo[c] = __funnelshift_r(g0.x, g1.x, sh); whi[c] = __funnelshift_r(g0.y, g1.y, sh);
+          }
         }
       }
       const int t = __shfl_sync(0xffffffffu, my_t, ph), mism = __shfl_sync(0xffffffffu, my_mism, ph);
-      const int qb = inside ? (int)(((wlo >> ph) & 1u) | (((whi >> ph) & 1u) << 1)) : 4;
-      int sco;
-      if (t == 4 || qb == 4) sco = -sc.n_pen;
-      else if (t == qb || (t == 3 && qb == 1)) sco = 0;
-      else sco = mism;
-      const int m = hd + sco;
-      int e = __shfl_down_sync(0xffffffffu, e_prev, 1);
-      if (i == 0) e = -goe; else if (lane == band - 1) e = NEG;
-      u32 d = m >= e ? 0u : 1u;
-      int h = m >= e ? m : e;
-      const int open = m - goe;
-      // f entering cell jj: NEG at the band start, then f[jj+1] = max(f[jj] - ge, open[jj]) -- a prefix maximum of open[q] + q ge
-      int a = act ? open + lane * ge : (int)0x80000000;
+      int carry = 0;                                    // the low half's scan maximum (lane 31), where the high half's scan starts
 #pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, a, o); if (lane >= o) a = max(a, v); }
-      const int ex = __shfl_up_sync(0xffffffffu, a, 1);
-      const int f = lane == 0 ? NEG : max(NEG - lane * ge, ex - (lane - 1) * ge);
-      d = h >= f ? d : 2u;
-      h = h >= f ? h : f;
-      e -= ge;
-      const bool e_ext = e > open;
-      if (!e_ext) e = open;
-      const bool f_ext = f - ge > open;
-      const u32 b0 = __ballot_sync(0xffffffffu, act && (d & 1u)), b1 = __ballot_sync(0xffffffffu, act && (d & 2u));
-      const u32 be = __ballot_sync(0xffffffffu, act && e_ext), bf = __ballot_sync(0xffffffffu, act && f_ext);
-      if (lane == 0) dir[i] = make_uint4(b0, b1, be, bf);
-      hd = h; e_prev = e;
+      for (int c = 0; c < C; ++c) {
+        const int jj = lane + 32 * c;
+        const int qb = inside ? (int)(((wlo[c] >> ph) & 1u) | (((whi[c] >> ph) & 1u) << 1)) : 4;
+        int sco;
+        if (t == 4 || qb == 4) sco = -sc.n_pen;
+        else if (t == qb || (t == 3 && qb == 1)) sco = 0;
+        else sco = mism;
+        const int m = hd[c] + sco;
+        // e entering cell jj comes from cell jj + 1 of the row above: lane 31 of the low half reads lane 0 of the high half, whose
+        // e_prev still holds the row above
+        int e = c + 1 < C ? __shfl_sync(0xffffffffu, lane == 0 ? e_prev[(c + 1) % C] : e_prev[c], lane + 1) : __shfl_down_sync(0xffffffffu, e_prev[c], 1);
+        if (i == 0) e = -goe; else if (jj == band - 1) e = NEG;
+        u32 d = m >= e ? 0u : 1u;
+        int h = m >= e ? m : e;
+        const int open = m - goe;
+        // f entering cell jj: NEG at the band start, then f[jj+1] = max(f[jj] - ge, open[jj]) -- a prefix maximum of open[q] + q ge
+        int a = act[c] ? open + jj * ge : (int)0x80000000;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, a, o); if (lane >= o) a = max(a, v); }
+        if (c > 0) a = max(a, carry);
+        int ex = __shfl_up_sync(0xffffffffu, a, 1);
+        if (c > 0 && lane == 0) ex = carry;
+        if (c + 1 < C) carry = __shfl_sync(0xffffffffu, a, 31);
+        const int f = jj == 0 ? NEG : max(NEG - jj * ge, ex - (jj - 1) * ge);
+        d = h >= f ? d : 2u;
+        h = h >= f ? h : f;
+        e -= ge;
+        const bool e_ext = e > open;
+        if (!e_ext) e = open;
+        const bool f_ext = f - ge > open;
+        const u32 b0 = __ballot_sync(0xffffffffu, act[c] && (d & 1u)), b1 = __ballot_sync(0xffffffffu, act[c] && (d & 2u));
+        const u32 be = __ballot_sync(0xffffffffu, act[c] && e_ext), bf = __ballot_sync(0xffffffffu, act[c] && f_ext);
+        if (lane == 0) dir[i * C + c] = make_uint4(b0, b1, be, bf);
+        hd[c] = h; e_prev[c] = e;
+      }
     }
     // best end in the last row: the middle of the band unless another cell is strictly better, then the rightmost best one
-    const int hv = act ? hd : (int)0x80000000;
+    int hv = (int)0x80000000;
+#pragma unroll
+    for (int c = 0; c < C; ++c) if (act[c]) hv = max(hv, hd[c]);
     const int vmax = __reduce_max_sync(0xffffffffu, hv);
-    const u32 at_max = __ballot_sync(0xffffffffu, act && hd == vmax);
-    const int best_lane = ((at_max >> k) & 1u) ? k : 31 - __clz((int)at_max);
+    u64 at_max = 0;
+#pragma unroll
+    for (int c = 0; c < C; ++c) at_max |= (u64)__ballot_sync(0xffffffffu, act[c] && hd[c] == vmax) << (32 * c);
+    const int best = C == 1 ? (((u32)at_max >> k) & 1u ? k : 31 - __clz((int)at_max))
+                            : ((at_max >> k) & 1u ? k : 63 - __clzll((long long)at_max));
     __syncwarp();
     if (lane == 0) {
       u32* ops = ops_scratch + ops_off[it];
@@ -1632,9 +1532,9 @@ __global__ void __launch_bounds__(32 * RW_WARPS) refine_warp(DevIndex ix, const 
       auto push = [&](u32 op, u32 len) {
         if (n_ops == 0 || (cur & 0xfu) != op) { if (n_ops) ops[cap - n_ops] = cur; cur = len << 4 | op; ++n_ops; } else cur += len << 4;
       };
-      int i = rlen - 1, j = rlen - 1 + best_lane, state = 0;
+      int i = rlen - 1, j = rlen - 1 + best, state = 0;
       while (i >= 0 && j >= 0) {
-        const uint4 dd = dir[i]; const int jj = j - i;
+        const uint4 dd = dir[C == 1 ? i : i * C + ((j - i) >> 5)]; const int jj = C == 1 ? j - i : (j - i) & 31;   // cell j - i's word and bit
         if (state == 0) state = (int)(((dd.x >> jj) & 1u) | (((dd.y >> jj) & 1u) << 1));
         else if (state == 1) state = (int)((dd.z >> jj) & 1u);
         else state = (int)(((dd.w >> jj) & 1u) << 1);
@@ -1644,7 +1544,7 @@ __global__ void __launch_bounds__(32 * RW_WARPS) refine_warp(DevIndex ix, const 
       }
       if (i >= 0) push(2, (u32)(i + 1));
       if (n_ops) ops[cap - n_ops] = cur;
-      int qb = j + 1, qe = rlen - 1 + best_lane, cb = 0, ce = -1;
+      int qb = j + 1, qe = rlen - 1 + best, cb = 0, ce = -1;
       if (n_ops) refine_fix_ends(ops + (cap - n_ops), (int)n_ops, qb, qe, cb, ce);
       s_fin[w][0] = qb; s_fin[w][1] = qe; s_fin[w][2] = (int)(cap - n_ops) + cb; s_fin[w][3] = ce - cb + 1;
     }
@@ -1963,7 +1863,7 @@ __global__ void finalize_reads(BatchView b) {
 //   * try_cigar_without_path (ksw.cpp:2515-2570): the best hit's diagonal re-read against the genome; exactly `err` mismatches
 //     on it = an ungapped alignment, CIGAR <L>M, and the mismatch positions go back so that the host can price them by quality
 //     (MismatchPenaltyByQuality; the quality strings never cross the link for such reads).  Otherwise the read is marked
-//     BMBS_FIN_DP: the banded affine DP (refine_dp) decides.
+//     BMBS_FIN_DP: the banded affine DP (refine_warp) decides.
 //   * coordinates (Schema.cpp:12596-12650, :9188-9244): strand, chromosome, 1-based POS, and the drop of hits that run over
 //     the end of their chromosome.
 struct FinCounters { unsigned long long mism_used, fb_used, n_sorted, n_host, n_dp, n_unc_idx, n_unc_sbd, n_long, cursor_long, cursor_sorted, n_huge, cursor_huge, pad[4]; };

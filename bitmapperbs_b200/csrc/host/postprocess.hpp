@@ -23,6 +23,7 @@
 #include <string>
 #include <vector>
 #include "../../../include/bmbs.h"
+#include "../bmbs_refine_ends.h"
 
 namespace bmbs {
 
@@ -283,29 +284,6 @@ struct DpQueue {
   }
 };
 
-// End fix-ups of fast_recalculate_bs_Cigar (ksw.cpp:2894-2990): the read is aligned end to end, so insertions at either end of
-// the traceback become matches and the window span grows with them.  ops[cb..ce] is what stays.
-inline void fix_ends(std::vector<uint32_t>& ops, int& qb, int& qe, int& cb, int& ce) {
-  const int n = (int)ops.size();
-  int i = 0, ins = 0;
-  for (; i < n && (ops[i] & 0xf) == 2; ++i) ins += ops[i] >> 4;
-  if (i != 0) {
-    uint32_t op = ops[i] & 0xf, len = ops[i] >> 4;   // (i == n cannot happen for a non-empty read with a match)
-    if (op == 0) len += ins; else { op = 0; len = ins; --i; }
-    ops[i] = len << 4 | op;
-    qb -= ins;
-  }
-  cb = i;
-  ins = 0;
-  for (i = n - 1; i >= cb && (ops[i] & 0xf) == 2; --i) ins += ops[i] >> 4;
-  if (i != n - 1) {
-    uint32_t op = ops[i] & 0xf, len = ops[i] >> 4;
-    if (op == 0) len += ins; else { op = 0; len = ins; ++i; }
-    ops[i] = len << 4 | op;
-    qe += ins;
-  }
-  ce = i;
-}
 // NM over the final operations (ksw.cpp:2990-3143): mismatches of the match runs (read T on window C is none) + gap lengths
 inline unsigned recount_nm(const char* win, const char* read, const std::vector<uint32_t>& ops, int cb, int ce, int qb) {
   unsigned nm = 0; int wi = qb, ri = 0;
@@ -354,7 +332,7 @@ inline void refine_alignment(const char* win, int wlen, const char* read, int rl
   else if (dq->mode == DpQueue::COLLECT) { dq->request(site, read, qual.data(), rlen, k); out.score = 0; out.start_site = end_site - rlen + 1; out.end_site = end_site; out.err = err; out.cigar = "*"; return; }   // placeholder, the unit is redone
   else { dq->take(forward, out); return; }       // the device returns the final operations: fix-ups and NM recount included
   int cb, ce;
-  fix_ends(ops, qb, qe, cb, ce);
+  refine_fix_ends(ops.data(), (int)ops.size(), qb, qe, cb, ce);
   const unsigned nm = recount_nm(win, read, ops, cb, ce, qb);
   char buf[32];
   for (int x = cb; x <= ce; ++x) {

@@ -23,7 +23,7 @@ def _newer(target: Path, sources) -> bool:
 
 def build(force=False):
     OUT.mkdir(exist_ok=True)
-    deps = sorted(HERE.glob("*.hpp")) + sorted((HERE.parent / "bitmapperbs_b200/csrc/host").glob("*.hpp"))
+    deps = sorted(HERE.glob("*.hpp")) + sorted((HERE.parent / "bitmapperbs_b200/csrc/host").glob("*.hpp")) + [HERE.parent / "bitmapperbs_b200/csrc/bmbs_refine_ends.h"]
     cli = OUT / "oracle_cli"
     if force or _newer(cli, [HERE / "oracle_cli.cpp", *deps]):
         subprocess.run(["g++", "-O2", "-std=c++17", "-Wall", "-Wno-sign-compare", str(HERE / "oracle_cli.cpp"), "-o", str(cli), "-lz"], check=True)

@@ -319,7 +319,7 @@ int orc_refine(const char* win, int wlen, const char* read, int rlen, int k, int
   return 0;
 }
 // the banded DP alone (banded_affine_align = ksw_semi_global_quality_back, ksw.cpp:1850-2045) on the window at `site`:
-// what the refine_dp kernel must reproduce value for value
+// what the refine_warp kernels must reproduce value for value
 int orc_banded_align(void* h, uint64_t site, const char* read, const char* qual, int rlen, int k, int mp_max, int mp_min, int n_pen, int gap_open,
                      int gap_ext, int q_base, int* score, int* qb, int* qe, uint32_t* ops, int ops_cap) {
   bmbs::Scoring sc; sc.mp_max = mp_max; sc.mp_min = mp_min; sc.n_pen = n_pen; sc.gap_open = gap_open; sc.gap_ext = gap_ext; sc.q_base = q_base;
@@ -334,7 +334,7 @@ int orc_banded_align(void* h, uint64_t site, const char* read, const char* qual,
 }
 
 // The whole refinement of an alignment with indels as the reference finishes it: the DP above, then the end fix-ups and the NM
-// recount (host/postprocess.hpp fix_ends / recount_nm, pinned to fast_recalculate_bs_Cigar by tests/test_refine_vs_reference.py).
+// recount (refine_fix_ends of csrc/bmbs_refine_ends.h and host/postprocess.hpp recount_nm, pinned to fast_recalculate_bs_Cigar by tests/test_refine_vs_reference.py).
 // What bmbs_refine returns is compared with this.  ops[] receives the final operations in read order.
 int orc_refine_final(void* h, uint64_t site, const char* read, const char* qual, int rlen, int k, int mp_max, int mp_min, int n_pen, int gap_open,
                      int gap_ext, int q_base, int* score, int* qb, int* qe, unsigned* nm, uint32_t* ops, int ops_cap) {
@@ -345,7 +345,7 @@ int orc_refine_final(void* h, uint64_t site, const char* read, const char* qual,
   std::vector<uint32_t> o;
   bmbs::banded_affine_align(win.data(), wlen, read, rlen, k, qual, sc, *score, *qb, *qe, o);
   int cb, ce;
-  bmbs::fix_ends(o, *qb, *qe, cb, ce);
+  bmbs::refine_fix_ends(o.data(), (int)o.size(), *qb, *qe, cb, ce);
   *nm = bmbs::recount_nm(win.data(), read, o, cb, ce, *qb);
   if (ce - cb + 1 > ops_cap) return -1;
   for (int i = cb; i <= ce; ++i) ops[i - cb] = o[i];

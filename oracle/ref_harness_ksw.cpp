@@ -1,7 +1,7 @@
 // oracle/ (test infrastructure): exposes the REFERENCE's own CIGAR refinement -- fast_recalculate_bs_Cigar (ksw.cpp:2578-3148)
 // with try_cigar_without_path (:2515-2570) and ksw_semi_global_quality_back (:1850-2045) -- through a C ABI, with the
 // substitution matrices set up as Prepare_alignment does (Schema.cpp:828-850).  Compiled by build_ref.sh from a scratch copy
-// of /root/reference; pins host/postprocess.hpp's refine_alignment (CPU) and the refine_dp kernel (GPU) for SURVEY.md 8f-1.
+// of /root/reference; pins host/postprocess.hpp's refine_alignment (CPU) and the refine_warp kernels (GPU) for SURVEY.md 8f-1.
 #include <cstdint>
 #include <cstring>
 #include "ksw.h"

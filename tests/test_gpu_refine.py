@@ -1,9 +1,9 @@
-"""GPU (-m gpu), SURVEY.md 8f-1: the refinement kernels behind bmbs_refine (refine_warp: a warp per alignment for bands of up
-to 32 cells; refine_dp: a thread per alignment for wider bands, and for every band with BMBS_REFINE_THREAD=1) against the CPU
-refinement (host/postprocess.hpp banded_affine_align + fix_ends + recount_nm, pinned to the reference's
+"""GPU (-m gpu), SURVEY.md 8f-1: the refinement kernels behind bmbs_refine (refine_warp<1>: a warp per alignment for bands of up
+to 32 cells, one cell per lane; refine_warp<2>: bands of 33..63 cells, two cells per lane) against the CPU refinement
+(host/postprocess.hpp banded_affine_align + refine_fix_ends + recount_nm, pinned to the reference's
 fast_recalculate_bs_Cigar by tests/test_refine_vs_reference.py): score, first / last window position, NM and every final
 operation identical, on windows of both strands, reads with substitutions, insertions, deletions and N, k up to 31, read
-lengths 30..640, windows that leave the strand, non-default scoring and phred64 qualities.  The whole-program SAM
+lengths 30..1000, windows that leave the strand, non-default scoring and phred64 qualities.  The whole-program SAM
 comparisons of test_gpu_parity.py cover the host glue around it."""
 import os
 import numpy as np
@@ -16,7 +16,7 @@ from oracle_binding import OracleIndex, refine_final
 pytestmark = pytest.mark.gpu
 
 
-# small_grid: refine_warp's grid sized for one SM (16 blocks of 4 warps), so that each warp takes many alignments in turn
+# small_grid: both refine_warp grids sized for one SM (16 blocks of 4 warps), so that each warp takes many alignments in turn
 GRIDS = {"default": {}, "small_grid": {"BMBS_GRID_SMS": "1"}}
 
 
@@ -83,21 +83,21 @@ def make_items(oidx, rng, n, lengths, scoring):
     return bytes(seqs), bytes(quals), items
 
 
-@pytest.mark.parametrize("thread_kernel", [0, 1])
+# 15 and 17: lengths 200 and 390 give k = 16 and k = 31, the narrowest and the widest band of refine_warp<2>; 16 and 17: wide
+# bands under non-default scoring and phred64; 18: reads of up to 1000 bases, the largest shared memory of both instances
 @pytest.mark.parametrize("seed,lengths,scoring", [(11, [100, 150], (6, 2, 1, 5, 3, 33)), (12, [30, 64, 250, 640], (6, 2, 1, 5, 3, 33)),
-                                                  (13, [100, 151], (4, 1, 2, 3, 1, 33)), (14, [125], (6, 2, 1, 5, 3, 64))])
-def test_refine_matches_cpu(gidx, oidx, seed, lengths, scoring, thread_kernel):
+                                                  (13, [100, 151], (4, 1, 2, 3, 1, 33)), (14, [125], (6, 2, 1, 5, 3, 64)),
+                                                  (15, [100, 200, 390], (6, 2, 1, 5, 3, 33)), (16, [120, 250, 300], (4, 1, 2, 3, 1, 33)),
+                                                  (17, [100, 200, 390], (6, 2, 1, 5, 3, 64)), (18, [150, 999, 1000], (6, 2, 1, 5, 3, 33))])
+def test_refine_matches_cpu(gidx, oidx, seed, lengths, scoring):
     rng = np.random.default_rng(seed)
     seqs, quals, items = make_items(oidx, rng, 1500, lengths, scoring)
     rf = B.Refiner(gidx)
-    if thread_kernel:
-        os.environ["BMBS_REFINE_THREAD"] = "1"
-    try:
-        res, ops = rf.refine(seqs, quals, items, scoring)
-    finally:
-        os.environ.pop("BMBS_REFINE_THREAD", None)
+    res, ops = rf.refine(seqs, quals, items, scoring)
     assert int(res["n_ops"].sum()) == len(ops)
-    assert (2 * items["k"].astype(int) + 1 <= 32).sum() > 300 and (2 * items["k"].astype(int) + 1 > 32).sum() > 50      # both kernels have work
+    band = 2 * items["k"].astype(int) + 1
+    assert (band <= 32).sum() > 300 and (band > 32).sum() > 50      # both band classes have work
+    assert (band == 33).any() and (band == 63).any()                # one cell in the high half, and the high half full
     for i, it in enumerate(items):
         o, L = int(it["seq_off"]), int(it["len"])
         score, qb, qe, nm, cops = refine_final(oidx, it["site"], seqs[o:o + L], quals[o:o + L], int(it["k"]), scoring)

@@ -1,10 +1,10 @@
 #!/usr/bin/env python3
-"""CIGAR refinement microbench (SURVEY.md 8f-1): n alignments of L = 150, k = 12 with one indel each through bmbs_refine
-(H2D of reads + qualities, refine_warp -- or refine_dp with BMBS_REFINE_THREAD=1 --, D2H of scores, NM and final operations),
-next to the same refinement on the host cores (host/postprocess.hpp through the oracle library, one thread).
-Cells = n * L * (2k + 1).
+"""CIGAR refinement microbench (SURVEY.md 8f-1): n alignments of length L and error threshold k (default L = 150, k = 12) with
+one indel each through bmbs_refine (H2D of reads + qualities, refine_warp<1> for k <= 15 or refine_warp<2> for k 16..31, D2H
+of scores, NM and final operations), next to the same refinement on the host cores (host/postprocess.hpp through the oracle
+library, one thread).  Cells = n * L * (2k + 1).
 
-  python tools/bench_refine.py [--n 131072]          (run under `ncu -k regex:refine_` for the kernel alone)
+  python tools/bench_refine.py [--n 131072] [--L 150] [--k 12]          (run under `ncu -k regex:refine_` for the kernel alone)
 """
 import argparse, gzip, json, shutil, subprocess, sys, tempfile, time
 from pathlib import Path
@@ -14,14 +14,15 @@ sys.path.insert(0, str(ROOT)); sys.path.insert(0, str(ROOT / "tests"))
 import bitmapperbs_b200 as B
 from bitmapperbs_b200 import capi
 
-ap = argparse.ArgumentParser(); ap.add_argument("--n", type=int, default=131072); ap.add_argument("--cpu-sample", type=int, default=2000); a = ap.parse_args()
+ap = argparse.ArgumentParser(); ap.add_argument("--n", type=int, default=131072); ap.add_argument("--cpu-sample", type=int, default=2000)
+ap.add_argument("--L", type=int, default=150); ap.add_argument("--k", type=int, default=12); a = ap.parse_args()
 with tempfile.TemporaryDirectory() as td:
     td = Path(td)
     with gzip.open(ROOT / "tests/golden/genome.fa.gz", "rb") as f, open(td / "genome.fa", "wb") as o:
         shutil.copyfileobj(f, o)
     subprocess.run([str(ROOT / "bitmapperbs_b200/_build/bmbs-index"), str(td / "genome.fa")], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     genome = np.frombuffer(b"".join(l.strip() for l in open(td / "genome.fa", "rb") if not l.startswith(b">")).upper(), dtype=np.uint8)
-    L, k, n = 150, 12, a.n
+    L, k, n = a.L, a.k, a.n
     rng = np.random.default_rng(1)
     sites = rng.integers(1000, len(genome) - 1000, size=n)
     reads = np.empty((n, L), dtype=np.uint8)
